@@ -2,6 +2,7 @@
 """bench.py -- PLEN env-steps/sec on B200 (BASELINE.json metric) with roofline, end-to-end and CPU-baseline legs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--total-envs T | --envs-per-gpu E] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one vectorised env step (1 action -> 4 physics ticks -> obs/reward/done/auto-reset) of every env of the
 rank: 3 launches per tick (k_dyn, k_rank, k_solve) + k_post (+ the rare-path k_solve_x).  Workload = BASELINE config 5
@@ -58,6 +59,9 @@ FLOP_PER_ENV_STEP = 4 * (FLOP_DYN_PER_ROBOT_TICK + FLOP_SOLVE_PER_ROBOT_TICK) + 
 # oracle's instrumented FLOP counter (plen_oracle_state.flops; scripts/oracle_flops.py): 1.32 Mflop per env-step
 REF_ALGO_FLOP_PER_ENV_STEP = 1.32e6
 FP32_NOMINAL_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12          # SURVEY.md section 8d
+# --dump-outputs: a step hands its caller 55 floats per env (obs 26, reward, done, timeout, terminal_obs 26), 220 bytes in
+# float32; at most this many envs are written (57.7 MB), a fixed seeded sample of them when the run has more
+DUMP_MAX_ENVS = 262144
 
 
 def _peaks():
@@ -204,6 +208,21 @@ def time_steps(env, acts, K, dev, flush=None):
     return tot / K
 
 
+def dump_index(n, dev):
+    """Envs whose outputs --dump-outputs writes: all n, or DUMP_MAX_ENVS of them drawn with numpy seed 0 (ascending env
+    index) when n is larger -- the same envs in every run of the same size."""
+    import torch
+    idx = np.arange(n) if n <= DUMP_MAX_ENVS else np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ENVS, replace=False))
+    return torch.from_numpy(idx).to(dev)
+
+
+def sample_step_outputs(step_out, idx):
+    """float32 device copies of the rows idx of what env.step returned (obs, reward, done, info)."""
+    obs, reward, done, info = step_out
+    out = {"obs": obs, "reward": reward, "done": done, "timeout": info["timeout"], "terminal_obs": info["terminal_obs"]}
+    return {k: v.index_select(0, idx).float() for k, v in out.items()}
+
+
 def td3_leg(dev, dist, rank, world, vector_steps=24, envs=16384, batch=4096, updates_per_step=2):
     """BASELINE configs 4 / 5, the learner side: 16,384 device-resident envs per GPU feeding a device replay ring, TD3
     updates (plen_td3_*: tcgen05 3xTF32 products, minibatch 4096 per GPU) between env steps, and -- at N > 1 -- the ONE
@@ -281,7 +300,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-td3-leg", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (obs, reward, done, timeout, terminal_obs; rank 0's envs) "
+                         "as DIR/<name>.npy in float32, for at most %d envs (a fixed seeded sample of larger runs)" % DUMP_MAX_ENVS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -317,6 +341,7 @@ def main():
     gen.manual_seed(env_seed(0, rank))
     acts = [torch.empty((E, 18), device=dev).uniform_(-1, 1, generator=gen) for _ in range(4)]
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device=dev)   # 256 MiB > 126 MB L2
+    dump_idx = dump_index(E, dev) if args.dump_outputs and rank == 0 else None
     env.reset()
     for w in range(W):
         env.step(acts[w % 4])
@@ -339,11 +364,13 @@ def main():
     for k in range(K):
         flush.zero_()
         ev[k][0].record()
-        env.step(acts[k % 4])
+        step_out = env.step(acts[k % 4])
         ev[k][1].record()
     barrier()
     t_w1 = time.time()
     launches1 = env.launches
+    # copied now: the env returns reused buffers, which the steps below overwrite
+    dump = sample_step_outputs(step_out, dump_idx) if dump_idx is not None else None
     # ---- per-kernel durations for the roofline: Kb MORE steps of the same workload, right behind the timed region and
     #      still under the clock sampler, with the library's CUDA-event brackets around every kernel.  They are not part of
     #      the timed region because a bracketed plen_step runs its kernels in the single-stream order (a kernel's duration
@@ -450,6 +477,11 @@ def main():
                               "single-stream order, the timed steps run as two concurrent ranges like any user call (DESIGN.md); "
                               "k_solve includes k_rank and the rare-path k_solve_x of the tick" % (Kb, bracketed_ms / Kb),
         }
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy())
+        del dump
     env.close()
     del env, acts, h_act, h_obs
     torch.cuda.empty_cache()

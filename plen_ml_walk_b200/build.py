@@ -30,7 +30,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if p.returncode != 0:
         raise RuntimeError("nvcc failed building libplen_b200.so")
     with open(os.path.join(HERE, "csrc", "ptxas_info.txt"), "w") as f:
-        # register / spill report of every kernel (tracked: reviewable without a build); compile times would only be noise
+        # register / spill report of every kernel; compile times would only be noise.  Not tracked by git: the kernel names
+        # of anonymous namespaces carry a hash of the build directory, so every checkout writes a different file
         f.write("".join(l for l in p.stderr.splitlines(True) if "Compile time" not in l))
     return OUT
 
