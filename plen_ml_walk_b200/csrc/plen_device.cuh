@@ -201,6 +201,13 @@ PLEN_DEV void load6(const float *row, float (&o)[6]) {
     const vec2 b = *reinterpret_cast<const vec2 *>(row + 4);
     o[0] = a.x; o[1] = a.y; o[2] = a.z; o[3] = a.w; o[4] = b.x; o[5] = b.y;
 }
+// ... and the store: STS.128 + STS.64
+PLEN_DEV void store6(float *row, float v0, float v1, float v2, float v3, float v4, float v5) {
+    vec4 a; a.x = v0; a.y = v1; a.z = v2; a.w = v3;
+    vec2 b; b.x = v4; b.y = v5;
+    *reinterpret_cast<vec4 *>(row) = a;
+    *reinterpret_cast<vec2 *>(row + 4) = b;
+}
 
 // per-warp shared scratch of k_dyn (floats); 16-byte aligned so that the 8-float rows can be read as vectors
 struct PLEN_ALIGN16 WarpScratch {
@@ -349,19 +356,17 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
     forward_kinematics(tab, lane, L.q, L.quat, Rw, pw);
 
     // ---- joint twist s = [a; m] about the base origin (world axes); base lanes carry the identity columns
-    float a[3] = {0, 0, 0}, m[3] = {0, 0, 0};
+    //      (every index compile-time: a lane-indexed a[lane] = 1 would put a and m in local memory)
+    float a[3], m[3];
+#pragma unroll
+    for (int k = 0; k < 3; k++) { a[k] = (lane == k) ? 1.0f : 0.0f; m[k] = (lane == 3 + k) ? 1.0f : 0.0f; }
     if (is_joint) {
         float ax[3] = {tab[(T_AXIS + 0) * 32 + lane], tab[(T_AXIS + 1) * 32 + lane], tab[(T_AXIS + 2) * 32 + lane]};
         mat3_vec(Rw, ax, a);
         cross(pw, a, m);
-    } else if (lane < 3) {
-        a[lane] = 1.0f;
-    } else if (lane < 6) {
-        m[lane - 3] = 1.0f;
     }
     if (lane < 24) {
-#pragma unroll
-        for (int k = 0; k < 3; k++) { ws.tw[lane][k] = a[k]; ws.tw[lane][3 + k] = m[k]; }
+        store6(ws.tw[lane], a[0], a[1], a[2], m[0], m[1], m[2]);
     }
 
     // ---- body inertia about the base origin, world axes: mass, h = m c, Ibar (xx yy zz xy xz yz)
@@ -391,8 +396,7 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
 
     // ---- spatial velocity of this lane's body: V = V0 + sum_{ancestors} s_j qd_j
     float V0[6];
-#pragma unroll
-    for (int k = 0; k < 6; k++) V0[k] = shfl(L.u, k);
+    load6(ws.st + W_U, V0);       // base velocity = u of lanes 0..5, still in the staged state record (two broadcast reads)
     float tv[6];   // own term s * u (joint lanes only)
 #pragma unroll
     for (int k = 0; k < 3; k++) { tv[k] = is_joint ? a[k] * L.u : 0.0f; tv[3 + k] = is_joint ? m[k] * L.u : 0.0f; }
@@ -525,8 +529,9 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
         fM[2] = Ic[4] * a[0] + Ic[5] * a[1] + Ic[2] * a[2] + t[2];
         cross(hc, a, t);
         fM[3] = mc * m[0] - t[0]; fM[4] = mc * m[1] - t[1]; fM[5] = mc * m[2] - t[2];
-    } else if (lane < 6) {
-        Cl = Ft[lane];
+    } else {
+#pragma unroll
+        for (int k = 0; k < 6; k++) Cl = (lane == k) ? Ft[k] : Cl;   // compile-time indices: Ft stays in registers
     }
     ws.cb[lane] = Cl;
 
@@ -560,16 +565,27 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
         for (int k = 0; k < 6; k++) Krow[k] = fM[k];
         warp_sync();
     }
-    // Gauss-Jordan across the lanes of each chain: Mrow -> row of A_c = M_cc^-1, Krow -> row of K_c = A_c M_c0
+    // Gauss-Jordan across the lanes of each chain: Mrow -> row of A_c = M_cc^-1, Krow -> row of K_c = A_c M_c0.
+    // The pivot row of step k is published by lane cs + k in its own 12-word slot of red (free until the Schur products
+    // below) and read back with three LDS.128 instead of twelve SHFL.  A slot is written once, so one warp_sync per step
+    // suffices; the 48-byte slot stride keeps the four chains' pivot rows in distinct banks.
 #pragma unroll
     for (int k = 0; k < 6; k++) {
         const bool act = is_joint && (cs + k <= ce);
-        const int src = act ? cs + k : lane;
+        if (off == k) {
+            float *dst = ws.red + 12 * lane;
+            store6(dst, Mrow[0], Mrow[1], Mrow[2], Mrow[3], Mrow[4], Mrow[5]);
+            store6(dst + 6, Krow[0], Krow[1], Krow[2], Krow[3], Krow[4], Krow[5]);
+        }
+        warp_sync();
         float pr[6], pk[6];
-#pragma unroll
-        for (int d = 0; d < 6; d++) pr[d] = shfl(Mrow[d], src);
-#pragma unroll
-        for (int d = 0; d < 6; d++) pk[d] = shfl(Krow[d], src);
+        {
+            const float *srcp = ws.red + 12 * (act ? cs + k : 6 + k);   // idle lanes read a valid slot and ignore it
+            const vec4 x0 = *reinterpret_cast<const vec4 *>(srcp), x1 = *reinterpret_cast<const vec4 *>(srcp + 4),
+                       x2 = *reinterpret_cast<const vec4 *>(srcp + 8);
+            pr[0] = x0.x; pr[1] = x0.y; pr[2] = x0.z; pr[3] = x0.w; pr[4] = x1.x; pr[5] = x1.y;
+            pk[0] = x1.z; pk[1] = x1.w; pk[2] = x2.x; pk[3] = x2.y; pk[4] = x2.z; pk[5] = x2.w;
+        }
         if (act) {
             const float inv = rcp_(pr[k]);
             if (off == k) {
@@ -587,6 +603,7 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
         }
     }
 
+    warp_sync();   // the last pivot rows are read before red is overwritten
     // ---- base Schur complement S = M00 - sum_l fM_l (x) K_l, via a conflict-free smem transpose-reduce
     {
         int idx = 0;
@@ -603,9 +620,10 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
     }
     // note: red[0..20] is written by lanes < 21 while other lanes may still read red[j*21 + lane] for j >= 6 only
     warp_sync();
-    // ---- S^-1 by Gauss-Jordan ACROSS lanes 0..5 (lane r owns row r; the pivot row is broadcast with six SHFL per step)
-    //      instead of every lane inverting the full 6 x 6 redundantly: ~150 warp instructions instead of ~450.  Same
-    //      elimination order and operations per entry as a serial in-place Gauss-Jordan without pivoting (S is SPD).
+    // ---- S^-1 by Gauss-Jordan ACROSS lanes 0..5 (lane r owns row r; lane k publishes the scaled pivot row of step k in
+    //      kk[k], free until the K rows are stored below, and every lane reads it back as two broadcast LDS) instead of
+    //      every lane inverting the full 6 x 6 redundantly: ~150 warp instructions instead of ~450.  Same elimination order
+    //      and operations per entry as a serial in-place Gauss-Jordan without pivoting (S is SPD).
     float R[6];     // lanes 0..5: row `lane` of S, then of S^-1 (other lanes: scratch)
     {
         // M00 = [[Ibar, hx],[hx^T, m 1]] of the whole robot
@@ -635,8 +653,13 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
         for (int k = 0; k < 6; k++) {
             const float inv = rcp_(R[k]);
             float P[6];     // row k after scaling: [.. R[j] inv .., inv at j = k, ..]
+            if (lane == k) {
 #pragma unroll
-            for (int j = 0; j < 6; j++) P[j] = shfl((j == k) ? inv : R[j] * inv, k);
+                for (int j = 0; j < 6; j++) P[j] = (j == k) ? inv : R[j] * inv;
+                store6(ws.kk[k], P[0], P[1], P[2], P[3], P[4], P[5]);
+            }
+            warp_sync();
+            load6(ws.kk[k], P);
             const float f = R[k];
             const bool piv = lane == k;
 #pragma unroll
@@ -648,10 +671,7 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
     }
     // S^-1 to every lane through shared memory (gg is free until the G rows are stored below)
     warp_sync();
-    if (lane < 6) {
-#pragma unroll
-        for (int k = 0; k < 6; k++) ws.gg[lane][k] = R[k];
-    }
+    if (lane < 6) store6(ws.gg[lane], R[0], R[1], R[2], R[3], R[4], R[5]);
     warp_sync();
     // G = K S^-1
     float G[6];
@@ -670,23 +690,22 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
         }
     }
     warp_sync();
-    if (lane < 24) {
-#pragma unroll
-        for (int k = 0; k < 6; k++) { ws.kk[lane][k] = is_joint ? Krow[k] : 0.0f; ws.gg[lane][k] = G[k]; }
-    }
+    if (lane < 24) store6(ws.kk[lane], is_joint ? Krow[0] : 0.0f, is_joint ? Krow[1] : 0.0f, is_joint ? Krow[2] : 0.0f,
+                          is_joint ? Krow[3] : 0.0f, is_joint ? Krow[4] : 0.0f, is_joint ? Krow[5] : 0.0f);
     warp_sync();
-    // ---- assemble M^-1 (this lane's row), stored column-major so later reads are conflict free.  One branch-free loop:
-    //      joint lanes take G . K_j (+ the limb block), base lanes (G = 0) the transposed -G entries and their row of S^-1
+    // ---- assemble M^-1 (this lane's row), stored column-major so later reads are conflict free: lanes < 24 their row of
+    //      the base columns (-G, or S^-1 on base lanes), joint lanes also the base rows of their own column (the transposed
+    //      -G: one STS.128 + STS.64) and G . K_j (+ the limb block) in the joint columns
     if (lane < 24) {
 #pragma unroll
         for (int k = 0; k < 6; k++) ws.minv[k][lane] = is_joint ? -G[k] : R[k];
-        const float *ggl = &ws.gg[0][is_joint ? 0 : lane];
+        if (is_joint) store6(ws.minv[lane], -G[0], -G[1], -G[2], -G[3], -G[4], -G[5]);
 #pragma unroll 6
         for (int j = 6; j < 24; j++) {
             float r6[6];
             load6(ws.kk[j], r6);
             const float s = G[0] * r6[0] + G[1] * r6[1] + G[2] * r6[2] + G[3] * r6[3] + G[4] * r6[4] + G[5] * r6[5];
-            ws.minv[j][lane] = is_joint ? s : -ggl[j * 8];
+            if (is_joint) ws.minv[j][lane] = s;
         }
         if (is_joint) {
 #pragma unroll
@@ -720,21 +739,31 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
         L.lam = (lane >= 24) ? ws.mlam[lane - 24] : L.lam;
     } else {
         const int i = lane - 24, f = (lane >= 28) ? 1 : 0;
-        const int src = cfg.foot_lane[f];
-        float Rf[9], pf[3];
-#pragma unroll
-        for (int k = 0; k < 9; k++) Rf[k] = shfl(Rw[k], src);
-#pragma unroll
-        for (int k = 0; k < 3; k++) pf[k] = shfl(pw[k], src);
+        // the two foot lanes publish their frame (Rw, pw) in 16 words of kk each (free until the Y stash below); the contact
+        // lanes read it back with three LDS.128 instead of twelve SHFL
+        const int fw = (lane == cfg.foot_lane[0]) ? 0 : ((lane == cfg.foot_lane[1]) ? 1 : -1);
+        if (fw >= 0) {
+            vec4 *dst = reinterpret_cast<vec4 *>(&ws.kk[0][0] + 16 * fw);
+            vec4 x;
+            x.x = Rw[0]; x.y = Rw[1]; x.z = Rw[2]; x.w = Rw[3]; dst[0] = x;
+            x.x = Rw[4]; x.y = Rw[5]; x.z = Rw[6]; x.w = Rw[7]; dst[1] = x;
+            x.x = Rw[8]; x.y = pw[0]; x.z = pw[1]; x.w = pw[2]; dst[2] = x;
+        }
+        warp_sync();
         bool in = false;
         if (lane >= 24) {
+            const vec4 *fr = reinterpret_cast<const vec4 *>(&ws.kk[0][0] + 16 * f);
+            const vec4 x0 = fr[0], x1 = fr[1], x2 = fr[2];
+            const float Rf[9] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w, x2.x}, pf[3] = {x2.y, x2.z, x2.w};
             const float *pt = cfg.foot_pts[f][i & 3];
             float w[3];
             mat3_vec(Rf, pt, w);
             w[0] += pf[0]; w[1] += pf[1]; w[2] += pf[2];
             const float dist = (L.pos[2] + w[2]) - cfg.hull_margin;
             in = dist <= cfg.foot_break[f];
-            ws.cp[i][0] = w[0]; ws.cp[i][1] = w[1]; ws.cp[i][2] = w[2] - cfg.hull_margin; ws.cp[i][3] = dist;
+            vec4 c4;
+            c4.x = w[0]; c4.y = w[1]; c4.z = w[2] - cfg.hull_margin; c4.w = dist;
+            *reinterpret_cast<vec4 *>(ws.cp[i]) = c4;
             const bool was = (L.man >> i) & 1u;
             if (!in || !was) L.lam = 0.0f;
         }
@@ -771,7 +800,9 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
     const bool ext = nx > 0;
 
     // ---- masked twists and operational columns Y_f = M^-1 Jfoot_f^T per foot with active contacts
-    float Y[2][6];
+    float Y[2][6], mb[6];     // mb: this lane's row of the base columns of M^-1, read once for both feet
+#pragma unroll
+    for (int k = 0; k < 6; k++) mb[k] = (man_new || ext) && lane < 24 ? ws.minv[k][lane] : 0.0f;
 #pragma unroll
     for (int f = 0; f < 2; f++) {
         const int fl = cfg.foot_lane[f], fcs = fl - 5;
@@ -780,7 +811,7 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
         // (a robot with box contacts always carries the right-foot twist: the box rows are expressed through it)
         if ((((man_new >> (4 * f)) & 0xFu) || (f == 0 && ext)) && lane < 24) {
 #pragma unroll
-            for (int k = 0; k < 6; k++) Y[f][k] = ws.minv[k][lane];
+            for (int k = 0; k < 6; k++) Y[f][k] = mb[k];
             for (int j = fcs; j <= fl; j++) {
                 const float w = ws.minv[j][lane];
                 float r6[6];
@@ -818,29 +849,42 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
     //      contact-row lanes through ws.st[W_SPARE ..]; it used to be twelve full-warp butterfly reductions (60 SHFL).
     ws.obs[lane] = vstar;                           // obs is free scratch in k_dyn (lanes >= 24 hold 0)
     if (lane < 24) {
-#pragma unroll
-        for (int k = 0; k < 6; k++) { ws.kk[lane][k] = Y[0][k]; ws.gg[lane][k] = Y[1][k]; }
+        store6(ws.kk[lane], Y[0][0], Y[0][1], Y[0][2], Y[0][3], Y[0][4], Y[0][5]);
+        store6(ws.gg[lane], Y[1][0], Y[1][1], Y[1][2], Y[1][3], Y[1][4], Y[1][5]);
     }
     warp_sync();
     if (man_new || ext) {
         if (lane < 12) {
             const int f = (lane >= 6) ? 1 : 0, k = lane - 6 * f, fl = cfg.foot_lane[f];
+            float vb[6];                                // v* of the base: two broadcast reads
+            load6(ws.obs, vb);
             float acc = 0.0f;
 #pragma unroll
-            for (int l = 0; l < 6; l++) acc += ws.tw[l][k] * ws.obs[l];
+            for (int l = 0; l < 6; l++) acc += ws.tw[l][k] * vb[l];
 #pragma unroll
             for (int l = 0; l < 6; l++) acc += ws.tw[fl - 5 + l][k] * ws.obs[fl - 5 + l];
             ws.st[W_SPARE + lane] = acc;
         }
-        // Lambda^-1[fa*6+a][fb*6+b] = Y_fb[a][b] + sum_{j in leg fa} s_j[a] Y_fb[j][b]
-        for (int e = lane; e < 144; e += 32) {
-            const int row = e / 12, col = e - 12 * row;
-            const int fa = row / 6, a6 = row - 6 * fa, fb = col / 6, b6 = col - 6 * fb;
+        // Lambda^-1[fa*6+a][fb*6+b] = Y_fb[a][b] + sum_{j in leg fa} s_j[a] Y_fb[j][b], summed in leg order.
+        // Lane fa*12 + col (lanes < 24) owns the six entries (fa*6 + a, col): Y_fb[j][b] is read once for all six, the twist
+        // rows of leg fa as one broadcast row read per joint.  (It was 4.5 entries per lane with two scalar reads per term.)
+        if (lane < 24) {
+            const int fa = (lane >= 12) ? 1 : 0, col = lane - 12 * fa, fb = (col >= 6) ? 1 : 0, b6 = col - 6 * fb;
             const float(*Yb)[8] = fb ? ws.gg : ws.kk;
-            float acc = Yb[a6][b6];
-            const int fl = cfg.foot_lane[fa];
-            for (int j = fl - 5; j <= fl; j++) acc += ws.tw[j][a6] * Yb[j][b6];
-            ws.lin[row][col] = acc;
+            const int j0 = cfg.foot_lane[fa] - 5;
+            float acc[6];
+#pragma unroll
+            for (int a = 0; a < 6; a++) acc[a] = Yb[a][b6];
+#pragma unroll
+            for (int t = 0; t < 6; t++) {
+                float s6[6];
+                load6(ws.tw[j0 + t], s6);
+                const float y = Yb[j0 + t][b6];
+#pragma unroll
+                for (int a = 0; a < 6; a++) acc[a] += s6[a] * y;
+            }
+#pragma unroll
+            for (int a = 0; a < 6; a++) ws.lin[6 * fa + a][col] = acc[a];
         }
         warp_sync();
     }
@@ -862,24 +906,42 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
             const float *b1 = ij ? &ws.minv[6][6 + i] : (ic ? &Ya[6][a6] : &ws.cb[0]);
             const int st1 = ij ? 32 : (ic ? 8 : 0);
             const bool on1 = ij || ic;
+            float sc[18];                               // the 18 broadcast scales as one LDS.64 + four LDS.128
+            {
+                const vec2 s2 = *reinterpret_cast<const vec2 *>(ws.obs + 6);
+                sc[0] = s2.x; sc[1] = s2.y;
+#pragma unroll
+                for (int q = 0; q < 4; q++) {
+                    const vec4 s4 = *reinterpret_cast<const vec4 *>(ws.obs + 8 + 4 * q);
+                    sc[2 + 4 * q] = s4.x; sc[3 + 4 * q] = s4.y; sc[4 + 4 * q] = s4.z; sc[5 + 4 * q] = s4.w;
+                }
+            }
 #pragma unroll
             for (int c = 0; c < 18; c++) {
                 const float v = b1[c * st1];
-                G[c * 32 + lane] = on1 ? v * ws.obs[6 + c] : 0.0f;
+                G[c * 32 + lane] = on1 ? v * sc[c] : 0.0f;
             }
         }
         {
-            // column c = 18 + 6 fb + b6:  joint rows Y_fb[6 + i][b6] (kk / gg are adjacent [24][8] arrays), twist rows
-            // Lambda^-1[fa 6 + a6][c - 18] when any contact is active
+            // column c = 18 + 6 fb + b6:  joint rows Y_fb[6 + i][b6], twist rows Lambda^-1[fa 6 + a6][c - 18] when any
+            // contact is active; six consecutive words per foot (the Lambda^-1 half of fb = 1 is only 8-byte aligned)
             const bool on2 = ij || (ic && (man_new || ext));
             const float *b2 = ij ? &ws.kk[6 + i][0] : (on2 ? &ws.lin[fa * 6 + a6][0] : &ws.cb[0]);
-            const int jump = ij ? (int)(&ws.gg[0][0] - &ws.kk[0][0]) - 6 : 0, st2 = on2 ? 1 : 0;
+            const float *b2b = ij ? &ws.gg[6 + i][0] : b2 + 6;
+            float v2[12];
+            {
+                float r6[6];
+                load6(b2, r6);
 #pragma unroll
-            for (int c = 18; c < 30; c++) {
-                const int fb = (c >= 24) ? 1 : 0;
-                const float v = b2[(c - 18) * st2 + (fb ? jump : 0)];
-                G[c * 32 + lane] = on2 ? v : 0.0f;
+                for (int k = 0; k < 6; k++) v2[k] = r6[k];
+#pragma unroll
+                for (int k = 0; k < 3; k++) {
+                    const vec2 x = *reinterpret_cast<const vec2 *>(b2b + 2 * k);
+                    v2[6 + 2 * k] = x.x; v2[7 + 2 * k] = x.y;
+                }
             }
+#pragma unroll
+            for (int c = 18; c < 30; c++) G[c * 32 + lane] = on2 ? v2[c - 18] : 0.0f;
         }
         // per-joint scalars in the same word order (entries >= 18 are zero)
         const int src = ij ? 6 + i : 0;
@@ -956,8 +1018,10 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
         if (lane >= 24) srec[SR_LAMC + q2] = (pb2 >= 0) ? lc : 0.0f;
     }
     if (lane < 6) srec[SR_BASE + lane] = vstar;
-    if (lane < 3) srec[SR_BASE + 6 + lane] = L.pos[lane];
-    if (lane < 4) srec[SR_BASE + 9 + lane] = L.quat[lane];
+    // base pose from the staged state record (the copy L.pos / L.quat came from): a lane-indexed L.pos[lane] would put L in
+    // local memory
+    if (lane < 3) srec[SR_BASE + 6 + lane] = ws.st[W_POS + lane];
+    if (lane < 4) srec[SR_BASE + 9 + lane] = ws.st[W_QUAT + lane];
     if (lane == 0) {
         srec[SR_BASE + 13] = (float)man_new;
         srec[SR_BASE + 14] = L.fric_s;            // k_solve scales mu_lateral / mu_spinning / mu_rolling ...
