@@ -40,6 +40,7 @@ extern "C" {
 #define PLEN_MAX_BOXES 32      /* box colliders besides the two feet (plen.urdf: torso + 30 links): one per lane of a warp */
 #define PLEN_MAX_BOX_POINTS 4  /* box-vs-ground contact points kept per robot and tick (the deepest ones) */
 #define PLEN_MAX_HULL 256      /* convex-hull vertices of a foot collider (plen.urdf feet: 209 each) */
+#define PLEN_BODIES 19         /* rigid bodies of the robot: the torso composite and the body each of the 18 joints moves */
 #define PLEN_MAN_WORDS 52      /* per-robot persistent sole manifold (sole_manifold = 1): [foot][point][local xyz | plane xyz] = 48
                                   floats, the two point counts, 2 spare */
 
@@ -163,7 +164,7 @@ int plen_step(plen_ctx *ctx, const float *actions_dev, float *obs_dev, float *re
  * and a stream synchronise.  This is the end-to-end path a PyBullet user would see.
  * Ordering contract: the call runs on the context's PRIVATE streams (the batch is pipelined in ranges).  It first waits
  * (cudaStreamWaitEvent) for the work the last plen_reset / plen_step / plen_set_state / plen_set_manifold / plen_set_env_scales /
- * plen_tick call queued on its caller stream, so `plen_reset(...); plen_step_host(...)` needs no synchronisation in between; it
+ * plen_set_env_mass / plen_tick call queued on its caller stream, so `plen_reset(...); plen_step_host(...)` needs no synchronisation in between; it
  * returns after its own streams have drained, so whatever the caller queues next is ordered after it.  (Work the caller
  * queued on a stream WITHOUT going through this library -- e.g. a torch kernel still writing the state through
  * plen_set_state's source buffer -- is the caller's to order.) */
@@ -194,6 +195,23 @@ int plen_set_manifold(plen_ctx *ctx, const float *man_dev, void *stream);
  * NULL leaves a column as it is; every scale is 1 after plen_create.  Takes effect from the next tick. */
 int plen_set_env_scales(plen_ctx *ctx, const float *friction_scale_dev, const float *motor_force_scale_dev,
                         const float *motor_gain_scale_dev, void *stream);
+
+/* Per-env mass randomisation (SURVEY.md 8f-3): a robot carrying a different battery, cables or a sensor board.
+ *   mass_scale_dev [N,PLEN_BODIES]  factor on the mass AND the rotational inertia of each body (uniform density scaling, centre
+ *                  of mass unchanged).  Body 0 is the torso composite; body 1 + j is the body moved by joint j (action order).
+ *                  The URDF links folded into each body: PlenModel.body_links (plen_ml_walk_b200/urdf_loader.py).
+ *   payload_dev    [N,4]  (m, x, y, z): a point mass of m kg without rotational inertia, rigidly attached at (x, y, z) in the
+ *                  torso body frame (the frame of qpos's base pose).
+ * NULL leaves a part as it is.  Until the first call every robot has scale 1 and payload 0, and the context holds no mass
+ * table at all (the first call allocates 128 bytes per robot); a robot with scale 1 and payload 0 steps bit-identically to a
+ * context that never called this.  Takes effect from the next tick.  Precondition: scales finite and > 0, m finite and >= 0,
+ * x y z finite; a violation produces non-finite states, which the numeric guard retires (plen_fault_count).
+ * Approximation, as for plen_set_env_scales: a reset (explicit or auto) restores the ONE snapshot settled under the nominal
+ * model at plen_create; the robot's own masses apply from its first tick after that. */
+int plen_set_env_mass(plen_ctx *ctx, const float *mass_scale_dev, const float *payload_dev, void *stream);
+/* The current values into [N,PLEN_BODIES] / [N,4] device buffers (either NULL to skip), stream-ordered.  Returns 1 when
+ * plen_set_env_mass was ever called on this context, 0 when not (the buffers then receive 1 and 0), < 0 on error. */
+int plen_get_env_mass(plen_ctx *ctx, float *mass_scale_dev, float *payload_dev, void *stream);
 
 /* Advance every env by n_ticks physics ticks with raw joint targets [N,18] (radians) and no env logic.
  * Replaces move_joints + p.stepSimulation (plen_env.py:746-753, :665-667); used by the parity tests. */

@@ -55,6 +55,7 @@ struct plen_ctx {
     float *d_man;    // [n][PLEN_MAN_WORDS] persistent sole manifolds (cfg.sole_manifold = 1; NULL otherwise)
     float *d_hull;   // [2][PLEN_MAX_HULL][3] hull vertices of the feet (ditto)
     float *d_scale;  // [n][4] per-robot scales: friction, servo force limit, servo gain, reserved (plen_set_env_scales; all 1)
+    float *d_mass;   // [n][MR_WORDS] per-robot body mass scales and torso payload (plen_set_env_mass; NULL until its first call)
     uint8_t *d_key;  // [n] contact-load sort key of the current tick (k_dyn -> k_rank)
     int *d_perm;     // [n_tiles * RANK_TILE] robots ordered by contact load inside each tile (k_rank -> k_solve)
     float *d_act, *d_obs, *d_rew;
@@ -106,11 +107,14 @@ __device__ __forceinline__ DynSmem &stage_table(const float *tab_g) {
 //   actions != NULL : agent-space actions of a new env step; the servo targets are derived (agent_to_env) and kept in tgt
 //   actions == NULL : tgt holds the targets already (NULL = zero targets, the reset pose)
 // 5 CTAs (20 warps) per SM: the register cap (<= 102) costs 16 B of spills outside the hot loops and measured +2.4 %
+// MASS = true: the robots' mass rows (mrow, [n][MR_WORDS]) scale their bodies and add the torso payload; the false instance is
+// the stock path, untouched by the option (launched whenever no mass row applies).
+template <bool MASS>
 __global__ void __launch_bounds__(DYN_WPC * 32, DYN_CTAS)
 k_dyn(const __grid_constant__ DevConfig dc, const __grid_constant__ EnvRanges er, const float *__restrict__ tab_g,
       const float *__restrict__ state, int n, const float *__restrict__ actions, float *__restrict__ tgt,
       float *__restrict__ srec, uint8_t *__restrict__ keys, float *dbg_minv, float *dbg_pos, float *dbg_rot,
-      const float *__restrict__ scale, float *__restrict__ srx, float *__restrict__ man) {
+      const float *__restrict__ scale, float *__restrict__ srx, float *__restrict__ man, const float *__restrict__ mrow) {
     // The 4 KB model table is staged with cp.async while every warp already fetches its robot's state record and targets:
     // the two latencies overlap instead of adding up (the table wait used to sit in front of everything).
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -132,20 +136,23 @@ k_dyn(const __grid_constant__ DevConfig dc, const __grid_constant__ EnvRanges er
     }
     vec4 sc; sc.x = sc.y = sc.z = sc.w = 1.0f;
     if (has && scale) sc = gld4(scale + 4 * (size_t)env);
+    float mw = 1.0f;
+    if (MASS && has) mw = gld(mrow + (size_t)env * MR_WORDS + lane);     // one 128-byte line per robot
     asm volatile("cp.async.wait_all;" ::: "memory");
     __syncthreads();
     if (!has) return;
     LaneState L;
     unpack_record(r0, r1, r2, ws, L, lane);
     L.fric_s = sc.x; L.motor_s = sc.y; L.kp_s = sc.z;
+    L.mass_w = mw;
     if (jl) {
         if (actions) { L.tgt = agent_target(dc, er, lane - 6, a_in); tgt[o] = L.tgt; }
         else L.tgt = a_in;
     }
     DebugOut dbg{dbg_minv ? dbg_minv + (size_t)env * 576 : nullptr, dbg_pos ? dbg_pos + (size_t)env * 72 : nullptr,
                  dbg_rot ? dbg_rot + (size_t)env * 216 : nullptr};
-    tick_dynamics(dc, sm.tab, ws, L, lane, srec + (size_t)env * SR_WORDS, keys + env, (dbg_minv || dbg_pos || dbg_rot) ? &dbg : nullptr,
-                  srx ? srx + (size_t)env * XR_WORDS : nullptr, man ? man + (size_t)env * PLEN_MAN_WORDS : nullptr);
+    tick_dynamics<MASS>(dc, sm.tab, ws, L, lane, srec + (size_t)env * SR_WORDS, keys + env, (dbg_minv || dbg_pos || dbg_rot) ? &dbg : nullptr,
+                        srx ? srx + (size_t)env * XR_WORDS : nullptr, man ? man + (size_t)env * PLEN_MAN_WORDS : nullptr);
 }
 
 // Robots are grouped by contact load before the solve: k_rank counting-sorts the keys k_dyn wrote inside tiles of
@@ -270,6 +277,30 @@ __global__ void k_set_scales(float *__restrict__ scale, int n, const float *fric
     if (fric) s[0] = fric[e];
     if (motor) s[1] = motor[e];
     if (kp) s[2] = kp[e];
+}
+
+// per-robot mass rows: body scales [n][PLEN_BODIES] into words 0 and 6..23, payload [n][4] into words 24..27; NULL leaves a part
+// as it is, `init` first writes unit rows (scale 1, payload 0, padding 1).  One thread per word.
+__global__ void k_set_mass(float *__restrict__ mrow, int n, const float *scale, const float *payload, int init) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)n * MR_WORDS) return;
+    const size_t e = i / MR_WORDS;
+    const int w = (int)(i % MR_WORDS);
+    const bool pay = w >= MR_PAYLOAD && w < MR_PAYLOAD + 4, body = w == 0 || (w >= 6 && w < MR_PAYLOAD);
+    if (init) mrow[i] = pay ? 0.0f : 1.0f;
+    if (scale && body) mrow[i] = scale[e * PLEN_BODIES + (w == 0 ? 0 : w - 5)];
+    if (payload && pay) mrow[i] = payload[e * 4 + (w - MR_PAYLOAD)];
+}
+
+// ... and back; unit values when the context has no mass rows
+__global__ void k_get_mass(const float *__restrict__ mrow, int n, float *scale, float *payload) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)n * MR_WORDS) return;
+    const size_t e = i / MR_WORDS;
+    const int w = (int)(i % MR_WORDS);
+    const bool pay = w >= MR_PAYLOAD && w < MR_PAYLOAD + 4, body = w == 0 || (w >= 6 && w < MR_PAYLOAD);
+    if (scale && body) scale[e * PLEN_BODIES + (w == 0 ? 0 : w - 5)] = mrow ? mrow[i] : 1.0f;
+    if (payload && pay) payload[e * 4 + (w - MR_PAYLOAD)] = mrow ? mrow[i] : 0.0f;
 }
 
 // After the last tick of an env step, one warp per robot: observation, done, reward, counters, auto-reset.
@@ -520,6 +551,18 @@ static const size_t SOLVE_X_SMEM = sizeof(float) * (PLEN_GS_WORDS + PLEN_XS_WORD
 static int dyn_grid(int n) { return (n + DYN_WPC - 1) / DYN_WPC; }
 static int rank_tiles(int n) { return (n + RANK_TILE - 1) / RANK_TILE; }
 
+// k_dyn over n robots; the MASS instance only when mass rows apply (mrow != NULL), the stock instance otherwise
+static void launch_dyn(plen_ctx *ctx, const float *state, int n, const float *actions, float *tgt, float *srec, uint8_t *key,
+                       float *dbg_minv, float *dbg_pos, float *dbg_rot, const float *scale, float *srx, float *man,
+                       const float *mrow, cudaStream_t st) {
+    if (mrow)
+        k_dyn<true><<<dyn_grid(n), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->dc, ctx->er, ctx->d_tab, state, n, actions, tgt, srec, key,
+                                                                dbg_minv, dbg_pos, dbg_rot, scale, srx, man, mrow);
+    else
+        k_dyn<false><<<dyn_grid(n), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->dc, ctx->er, ctx->d_tab, state, n, actions, tgt, srec, key,
+                                                                 dbg_minv, dbg_pos, dbg_rot, scale, srx, man, nullptr);
+}
+
 // n_ticks physics ticks of 1/240 s: (k_dyn, k_solve) per tick.  `actions` (agent space) only on the first tick.
 // ev (nullable): 2*n_ticks events recorded before each kernel.
 static void launch_ticks(plen_ctx *ctx, float *state, int n, const float *actions, float *tgt, int n_ticks, cudaStream_t st,
@@ -534,11 +577,13 @@ static void launch_ticks(plen_ctx *ctx, float *state, int n, const float *action
     int *xg = boxes ? ctx->d_xgroups + off / RANK_TILE : nullptr;
     // persistent sole manifolds: the snapshot robot keeps its own behind its record
     float *man = !ctx->d_man ? nullptr : (state == ctx->d_snapshot ? ctx->d_snapshot + PLEN_SNAP_MAN : ctx->d_man + off * PLEN_MAN_WORDS);
+    // per-robot scales and mass rows: never for the snapshot robot, which is settled under the nominal parameters
+    const bool snap = state == ctx->d_snapshot;
+    const float *scale = (snap || !ctx->d_scale) ? nullptr : ctx->d_scale + 4 * off;
+    const float *mrow = (snap || !ctx->d_mass) ? nullptr : ctx->d_mass + MR_WORDS * off;
     for (int t = 0; t < n_ticks; t++) {
         if (ev) cudaEventRecord(ev[2 * t], st);
-        k_dyn<<<dyn_grid(n), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->dc, ctx->er, ctx->d_tab, state, n, t == 0 ? actions : nullptr,
-                                                          tgt, srec, key, nullptr, nullptr, nullptr,
-                                                          (state == ctx->d_snapshot || !ctx->d_scale) ? nullptr : ctx->d_scale + 4 * off, srx, man);
+        launch_dyn(ctx, state, n, t == 0 ? actions : nullptr, tgt, srec, key, nullptr, nullptr, nullptr, scale, srx, man, mrow, st);
         if (ev) cudaEventRecord(ev[2 * t + 1], st);
         const int nt = rank_tiles(n);
         k_rank<<<nt, RANK_TILE, 0, st>>>(key, n, perm, xg);
@@ -598,7 +643,7 @@ unsigned long long plen_kernel_launches(const plen_ctx *ctx) { return ctx ? ctx-
 void plen_destroy(plen_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    cudaFree(ctx->d_tab); cudaFree(ctx->d_state); cudaFree(ctx->d_snapshot); cudaFree(ctx->d_srec); cudaFree(ctx->d_srx); cudaFree(ctx->d_xgroups); cudaFree(ctx->d_tgt); cudaFree(ctx->d_key); cudaFree(ctx->d_perm); cudaFree(ctx->d_scale); cudaFree(ctx->d_man); cudaFree(ctx->d_hull);
+    cudaFree(ctx->d_tab); cudaFree(ctx->d_state); cudaFree(ctx->d_snapshot); cudaFree(ctx->d_srec); cudaFree(ctx->d_srx); cudaFree(ctx->d_xgroups); cudaFree(ctx->d_tgt); cudaFree(ctx->d_key); cudaFree(ctx->d_perm); cudaFree(ctx->d_scale); cudaFree(ctx->d_mass); cudaFree(ctx->d_man); cudaFree(ctx->d_hull);
     cudaFree(ctx->d_act); cudaFree(ctx->d_obs); cudaFree(ctx->d_rew); cudaFree(ctx->d_done); cudaFree(ctx->d_tmo); cudaFree(ctx->d_faults);
     for (int k = 1; k < PLEN_HOST_PIPE; k++)
         if (ctx->pipe[k]) cudaStreamDestroy(ctx->pipe[k]);
@@ -628,7 +673,8 @@ static int create_impl(plen_ctx *ctx) {
         }
     }
     CK(ctx, cudaSetDevice(ctx->device));
-    CK(ctx, cudaFuncSetAttribute(k_dyn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
+    CK(ctx, cudaFuncSetAttribute(k_dyn<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
+    CK(ctx, cudaFuncSetAttribute(k_dyn<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_post, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_observe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_solve<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_SMEM));
@@ -638,7 +684,8 @@ static int create_impl(plen_ctx *ctx) {
     CK(ctx, cudaFuncSetAttribute(k_solve_x, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     // both hot kernels are occupancy-limited by shared memory: ask for the largest carve-out (7 k_solve CTAs per SM)
     CK(ctx, cudaFuncSetAttribute(k_solve<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    CK(ctx, cudaFuncSetAttribute(k_dyn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    CK(ctx, cudaFuncSetAttribute(k_dyn<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    CK(ctx, cudaFuncSetAttribute(k_dyn<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     CK(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     ctx->pipe[0] = ctx->stream;
     for (int k = 1; k < PLEN_HOST_PIPE; k++) CK(ctx, cudaStreamCreateWithFlags(&ctx->pipe[k], cudaStreamNonBlocking));
@@ -808,7 +855,8 @@ int plen_step_host(plen_ctx *ctx, const float *actions_host, float *obs_host, fl
         const size_t off = bound[used], cnt = bound[used + 1] - off;
         cudaStream_t st = ctx->pipe[used % PLEN_HOST_PIPE];
         // ordering contract (plen_b200.h): this call runs on the context's private streams, so it first waits for whatever
-        // the last stream-taking entry point (reset / step / set_state / set_env_scales / tick) queued on the caller's stream
+        // the last stream-taking entry point (reset / step / set_state / set_env_scales / set_env_mass / tick) queued on the
+        // caller's stream
         CK(ctx, cudaStreamWaitEvent(st, ctx->last_work, 0));
         CK(ctx, cudaMemcpyAsync(ctx->d_act + off * PLEN_NJ, actions_host + off * PLEN_NJ, sizeof(float) * PLEN_NJ * cnt,
                                 cudaMemcpyHostToDevice, st));
@@ -833,6 +881,27 @@ int plen_set_env_scales(plen_ctx *ctx, const float *friction_scale_dev, const fl
     CK(ctx, cudaGetLastError());
     CK(ctx, mark_work(ctx, (cudaStream_t)stream));
     return PLEN_OK;
+}
+
+int plen_set_env_mass(plen_ctx *ctx, const float *mass_scale_dev, const float *payload_dev, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    CK(ctx, cudaSetDevice(ctx->device));
+    const size_t words = (size_t)MR_WORDS * ctx->n;
+    const int init = !ctx->d_mass;          // the rows are allocated at the first call: a context that never sets them has none
+    if (init) CK(ctx, cudaMalloc(&ctx->d_mass, sizeof(float) * words));
+    k_set_mass<<<(unsigned)((words + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ctx->d_mass, ctx->n, mass_scale_dev, payload_dev, init);
+    CK(ctx, cudaGetLastError());
+    CK(ctx, mark_work(ctx, (cudaStream_t)stream));
+    return PLEN_OK;
+}
+
+int plen_get_env_mass(plen_ctx *ctx, float *mass_scale_dev, float *payload_dev, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    CK(ctx, cudaSetDevice(ctx->device));
+    const size_t words = (size_t)MR_WORDS * ctx->n;
+    k_get_mass<<<(unsigned)((words + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ctx->d_mass, ctx->n, mass_scale_dev, payload_dev);
+    CK(ctx, cudaGetLastError());
+    return ctx->d_mass ? 1 : 0;
 }
 
 int plen_get_manifold(plen_ctx *ctx, float *man_dev, void *stream) {
@@ -893,9 +962,8 @@ int plen_tick(plen_ctx *ctx, const float *targets_dev, int n_ticks, void *stream
 int plen_debug_dynamics(plen_ctx *ctx, float *minv_dev, float *pos_dev, float *rot_dev, void *stream) {
     if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
-    k_dyn<<<dyn_grid(ctx->n), DYN_WPC * 32, DYN_SMEM, (cudaStream_t)stream>>>(ctx->dc, ctx->er, ctx->d_tab, ctx->d_state, ctx->n,
-                                                                            nullptr, nullptr, ctx->d_srec, ctx->d_key, minv_dev, pos_dev, rot_dev, ctx->d_scale, ctx->d_srx,
-                                                                            nullptr /* diagnostics must not advance the manifolds */);
+    launch_dyn(ctx, ctx->d_state, ctx->n, nullptr, nullptr, ctx->d_srec, ctx->d_key, minv_dev, pos_dev, rot_dev, ctx->d_scale, ctx->d_srx,
+               nullptr /* diagnostics must not advance the manifolds */, ctx->d_mass, (cudaStream_t)stream);
     CK(ctx, cudaGetLastError());
     return PLEN_OK;
 }

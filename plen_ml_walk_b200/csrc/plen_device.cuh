@@ -239,7 +239,12 @@ struct LaneState {
     int iters;        // PGS iterations of the last tick (diagnostic, uniform)
     float fric_s, motor_s, kp_s;   // per-robot scales of the friction coefficients, the servo force limit and the servo
                                    // gain (domain randomisation, plen_set_env_scales; 1 = the reference's constants)
+    float mass_w;     // word `lane` of the robot's mass row (plen_set_env_mass; read by the MASS instance of tick_dynamics
+                      // only): the mass scale of this lane's body (lanes 0, 6..23), the torso payload (lanes 24..27: m, x, y, z)
 };
+
+// per-robot mass row (plen_set_env_mass): 32 words, one per lane, so that a warp reads it with one 128-byte load
+enum { MR_PAYLOAD = 24, MR_WORDS = 32 };
 
 PLEN_DEV void mat3_mul(const float *A, const float *B, float *C) {
 #pragma unroll
@@ -347,6 +352,9 @@ PLEN_DEV_NOINLINE unsigned sole_manifold_contacts(const DevConfig &cfg, WarpScra
                                                   float pos2, float lam_in, float R0, float R1, float R2, float R3, float R4, float R5,
                                                   float R6, float R7, float R8, float p0, float p1, float p2);
 
+// MASS = true: the robot's own body masses and torso payload (L.mass_w) replace the model table's inertial values; the
+// false instance is the stock path and never reads L.mass_w.
+template <bool MASS = false>
 PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch &ws, LaneState &L, int lane,
                             float *srec, uint8_t *sort_key, const DebugOut *dbg = nullptr, float *srx = nullptr,
                             float *man = nullptr) {
@@ -370,16 +378,22 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
     }
 
     // ---- body inertia about the base origin, world axes: mass, h = m c, Ibar (xx yy zz xy xz yz)
-    const float mass = tab[T_MASS * 32 + lane];
+    float mass = tab[T_MASS * 32 + lane];
     float h[3], Ib[6];
     {
         float com[3] = {tab[(T_COM + 0) * 32 + lane], tab[(T_COM + 1) * 32 + lane], tab[(T_COM + 2) * 32 + lane]};
         float c[3];
         mat3_vec(Rw, com, c);
         c[0] += pw[0]; c[1] += pw[1]; c[2] += pw[2];
-        const float ixx = tab[(T_INERTIA + 0) * 32 + lane], iyy = tab[(T_INERTIA + 1) * 32 + lane],
-                    izz = tab[(T_INERTIA + 2) * 32 + lane], ixy = tab[(T_INERTIA + 3) * 32 + lane],
-                    ixz = tab[(T_INERTIA + 4) * 32 + lane], iyz = tab[(T_INERTIA + 5) * 32 + lane];
+        float ixx = tab[(T_INERTIA + 0) * 32 + lane], iyy = tab[(T_INERTIA + 1) * 32 + lane],
+              izz = tab[(T_INERTIA + 2) * 32 + lane], ixy = tab[(T_INERTIA + 3) * 32 + lane],
+              ixz = tab[(T_INERTIA + 4) * 32 + lane], iyz = tab[(T_INERTIA + 5) * 32 + lane];
+        if (MASS) {
+            // uniform density scaling of this lane's body: mass and rotational inertia times s, centre of mass unchanged
+            // (lanes >= 24 hold payload words, not scales; their table mass is 0 like that of lanes 1..5)
+            const float s = lane < MR_PAYLOAD ? L.mass_w : 1.0f;
+            mass *= s; ixx *= s; iyy *= s; izz *= s; ixy *= s; ixz *= s; iyz *= s;
+        }
         // Iw = Rw I Rw^T
         float T[9] = {Rw[0] * ixx + Rw[1] * ixy + Rw[2] * ixz, Rw[0] * ixy + Rw[1] * iyy + Rw[2] * iyz, Rw[0] * ixz + Rw[1] * iyz + Rw[2] * izz,
                       Rw[3] * ixx + Rw[4] * ixy + Rw[5] * ixz, Rw[3] * ixy + Rw[4] * iyy + Rw[5] * iyz, Rw[3] * ixz + Rw[4] * iyz + Rw[5] * izz,
@@ -392,6 +406,26 @@ PLEN_DEV void tick_dynamics(const DevConfig &cfg, const float *tab, WarpScratch 
         Ib[4] = T[0] * Rw[6] + T[1] * Rw[7] + T[2] * Rw[8] - mass * c[0] * c[2];
         Ib[5] = T[3] * Rw[6] + T[4] * Rw[7] + T[5] * Rw[8] - mass * c[1] * c[2];
         h[0] = mass * c[0]; h[1] = mass * c[1]; h[2] = mass * c[2];
+        if (MASS) {
+            // torso payload: a point mass m_p rigidly attached at r (torso body frame), added to lane 0's body with the same
+            // expressions.  Skipped for m_p = 0, so that a unit row leaves every bit as the stock path computes it.
+            const float mp = shfl(L.mass_w, MR_PAYLOAD);
+            const float r[3] = {shfl(L.mass_w, MR_PAYLOAD + 1), shfl(L.mass_w, MR_PAYLOAD + 2), shfl(L.mass_w, MR_PAYLOAD + 3)};
+            if (lane == 0 && mp != 0.0f) {
+                float cp[3];
+                mat3_vec(Rw, r, cp);
+                cp[0] += pw[0]; cp[1] += pw[1]; cp[2] += pw[2];
+                const float pp = cp[0] * cp[0] + cp[1] * cp[1] + cp[2] * cp[2];
+                mass += mp;
+                Ib[0] += mp * (pp - cp[0] * cp[0]);
+                Ib[1] += mp * (pp - cp[1] * cp[1]);
+                Ib[2] += mp * (pp - cp[2] * cp[2]);
+                Ib[3] -= mp * cp[0] * cp[1];
+                Ib[4] -= mp * cp[0] * cp[2];
+                Ib[5] -= mp * cp[1] * cp[2];
+                h[0] += mp * cp[0]; h[1] += mp * cp[1]; h[2] += mp * cp[2];
+            }
+        }
     }
 
     // ---- spatial velocity of this lane's body: V = V0 + sum_{ancestors} s_j qd_j

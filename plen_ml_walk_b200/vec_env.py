@@ -224,11 +224,64 @@ class PlenVecEnv:
         with torch.cuda.device(self.device):
             self._check(self.lib.plen_set_env_scales(self._ctx, *[self._p(x) for x in arr], self._stream()))
 
+    @property
+    def body_links(self):
+        """Names of the URDF links folded into each of the 19 bodies of set_env_mass: body 0 is the torso composite, body 1 + j
+        the body moved by joint j (action order)."""
+        return [list(self.model.body_links[0])] + [list(self.model.body_links[l]) for l in range(6, 24)]
+
+    def set_env_mass(self, mass_scale=None, payload=None):
+        """Per-env mass randomisation (SURVEY.md 8f-3).  None leaves a part unchanged.
+
+        mass_scale: [N] (one factor for every body) or [N,19]: factor on the mass and the rotational inertia of each body
+                    (uniform density scaling, centre of mass unchanged); the bodies are listed in body_links.
+        payload:    [N,4] (m, x, y, z): a point mass of m kg rigidly attached at (x, y, z) in the torso body frame (the frame of
+                    the base pose in get_state's qpos), without rotational inertia of its own.
+        Raises ValueError on a wrong shape, a scale that is not finite and > 0, or a payload that is not finite or has m < 0.
+        Before the first call every robot has scale 1 and payload 0, and such a robot steps bit-identically to a context that
+        never called this.  Takes effect from the next tick.
+
+        Approximation, as for set_env_scales: a reset (explicit or in-kernel auto-reset) restores the ONE post-reset snapshot
+        settled under the nominal model at creation; the robot's own masses apply from its first tick after that."""
+        n = self.num_envs
+        s = p = None
+        if mass_scale is not None:
+            s = torch.as_tensor(mass_scale, dtype=torch.float32, device=self.device)
+            if tuple(s.shape) == (n,):
+                s = s[:, None].expand(n, _abi.BODIES)
+            s = self._dev_f32(s, (n, _abi.BODIES))
+            if not bool(torch.isfinite(s).all()) or not bool((s > 0).all()):
+                raise ValueError("mass_scale must be finite and > 0")
+        if payload is not None:
+            p = self._dev_f32(payload, (n, 4))
+            if not bool(torch.isfinite(p).all()) or not bool((p[:, 0] >= 0).all()):
+                raise ValueError("payload must be finite with a mass >= 0")
+        with torch.cuda.device(self.device):
+            self._check(self.lib.plen_set_env_mass(self._ctx, self._p(s), self._p(p), self._stream()))
+
+    def _get_env_mass(self):
+        n, dev = self.num_envs, self.device
+        s = torch.empty((n, _abi.BODIES), dtype=torch.float32, device=dev)
+        p = torch.empty((n, 4), dtype=torch.float32, device=dev)
+        with torch.cuda.device(self.device):
+            rc = self.lib.plen_get_env_mass(self._ctx, self._p(s), self._p(p), self._stream())
+        if rc < 0:
+            self._check(rc)
+        return s, p, rc == 1
+
+    def get_env_mass(self):
+        """-> (mass_scale [N,19], payload [N,4]) as the device holds them (1 and 0 where set_env_mass was never called)."""
+        s, p, _ = self._get_env_mass()
+        return s, p
+
     def save_state(self, path):
-        """Snapshot of every env (pose, velocities, contact cache, env bookkeeping) to one .pt file (SURVEY.md 8f-4)."""
+        """Snapshot of every env (pose, velocities, contact cache, env bookkeeping, per-env scales and masses) to one .pt file
+        (SURVEY.md 8f-4)."""
         qpos, qvel, aux = self.get_state()
+        ms, mp, mass_set = self._get_env_mass()
         torch.save({"num_envs": self.num_envs, "joint_act": self.joint_act, "qpos": qpos.cpu(), "qvel": qvel.cpu(), "aux": aux.cpu(),
                     "scales": {k: v.cpu() for k, v in self._scales.items()},
+                    "mass": {"scale": ms.cpu(), "payload": mp.cpu()} if mass_set else None,
                     "manifold": self.get_manifold().cpu() if int(self.cfg.sole_manifold) else None}, path)
 
     def load_state(self, path):
@@ -243,6 +296,11 @@ class PlenVecEnv:
         if sc or self._scales:      # per-env scales travel with the snapshot; a snapshot without any restores the unit scales
             ones = torch.ones(self.num_envs)
             self.set_env_scales(*[sc.get(k, ones) for k in ("friction", "motor_force", "motor_gain")])
+        mass = d.get("mass")
+        if mass is not None:        # per-env masses likewise; a snapshot without them restores unit values if the context had some
+            self.set_env_mass(mass["scale"], mass["payload"])
+        elif self._get_env_mass()[2]:
+            self.set_env_mass(torch.ones(self.num_envs, _abi.BODIES), torch.zeros(self.num_envs, 4))
 
     def tick(self, targets, n_ticks=1):
         """Raw physics: n_ticks of 1/240 s with joint targets in radians, no env logic (move_joints + stepSimulation)."""

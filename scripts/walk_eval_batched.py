@@ -9,6 +9,10 @@ rollout (reset and policy are deterministic, so every noise-free env is identica
 noise to give a distribution.  Reports episode length / return of the first episode and the distance walked.
 
     python scripts/walk_eval_batched.py [--envs 4096] [--sigma 0.05] [--precision fp32|fp16]
+                                        [--mass-scale S] [--payload KG [--payload-offset X Y Z]]
+
+--mass-scale / --payload sweep the policy's robustness to the robot's mass (PlenVecEnv.set_env_mass): every body x S, and a
+point mass of KG kg on the torso, by default at the torso body's centre of mass.
 """
 import argparse
 import json
@@ -35,6 +39,10 @@ def main():
                     help="plen_config.sole_manifold: 1 = Bullet's one-point-per-tick persistent manifold (profiles/r2_physics_pin.md 5)")
     ap.add_argument("--config", action="append", default=[], metavar="KEY=VALUE",
                     help="plen_config override (repeatable), e.g. --config warmstart_factor=0.85 --config support_tie=0")
+    ap.add_argument("--mass-scale", type=float, default=None, help="factor on the mass and inertia of every body")
+    ap.add_argument("--payload", type=float, default=None, metavar="KG", help="point mass on the torso, kg")
+    ap.add_argument("--payload-offset", type=float, nargs=3, default=None, metavar=("X", "Y", "Z"),
+                    help="where the payload sits in the torso body frame, m (default: the torso's centre of mass)")
     a = ap.parse_args()
     dev = torch.device("cuda:0")
     g = np.load(GOLD)
@@ -46,6 +54,12 @@ def main():
         k, v = kv.split("=", 1)
         ovr[k] = float(v) if ("." in v or "e" in v.lower()) else int(v)
     env = PlenVecEnv(n, device=dev, auto_reset=False, config_overrides=ovr)
+    mass = None
+    if a.mass_scale is not None or a.payload is not None:
+        at = list(a.payload_offset) if a.payload_offset is not None else [float(v) for v in env.model.com[0]]
+        pay = torch.tensor([a.payload or 0.0] + at, dtype=torch.float32).expand(n, 4)
+        env.set_env_mass(None if a.mass_scale is None else torch.full((n,), a.mass_scale), pay if a.payload is not None else None)
+        mass = {"mass_scale": a.mass_scale, "payload_kg": a.payload, "payload_at_m": at if a.payload is not None else None}
     state = env.reset().clone()
     alive = torch.ones(n, dtype=torch.bool, device=dev)
     ep_len = torch.zeros(n, device=dev); ep_ret = torch.zeros(n, device=dev)
@@ -64,7 +78,7 @@ def main():
     L, R, X = ep_len.cpu().numpy(), ep_ret.cpu().numpy(), x_end.cpu().numpy()
     print(json.dumps({
         "policy": "plen_walk_gazebo_3229999 (reference checkpoint)", "envs": n, "steps": a.steps, "sigma": a.sigma,
-        "precision": a.precision, "sole_manifold": a.sole_manifold, "config_overrides": ovr,
+        "precision": a.precision, "sole_manifold": a.sole_manifold, "config_overrides": ovr, "mass": mass,
         "deterministic": {"episode_length": float(L[0]), "return": float(R[0]), "x_final_m": float(X[0])},
         "noisy": {"episode_length_mean": float(L[1:].mean()), "episode_length_median": float(np.median(L[1:])),
                   "survived_all_steps_frac": float((L[1:] >= a.steps).mean()), "return_mean": float(R[1:].mean()),
