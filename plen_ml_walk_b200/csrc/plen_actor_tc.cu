@@ -6,6 +6,8 @@
 // parity path (1e-5 against the reference's fp32 checkpoints), this one is the throughput path for rollouts
 // (FP16 operands, 11-bit significands: on the shipped checkpoint mean action error 4.5e-4, max 0.12 against fp32, bound
 // stated and tested in tests/test_td3_gpu.py; BF16 operands measured mean 4.2e-3 / max 0.59 there and were dropped).
+// Against a float64 model that rounds where this kernel rounds, the residual is the accumulation order alone: median 6e-14,
+// 99.9th percentile 4.8e-4 on the shipped checkpoint (tests/test_td3_kernels_gpu.py).
 //
 // One persistent CTA per SM, 128 threads, M = 128 observations per tile:
 //   * all three weight matrices live in shared memory as FP16 for the whole kernel (W2 128 KB, W1 / W3 16 KB each, K

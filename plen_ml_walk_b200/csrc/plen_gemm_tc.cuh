@@ -10,6 +10,9 @@
 //     x = hi + lo,   hi = rna_tf32(x),   lo = rna_tf32(x - hi),
 // and each product is accumulated as  A_lo B_hi + A_hi B_lo + A_hi B_hi  (the dropped A_lo B_lo term is 2^-22 relative):
 // fp32-level accuracy from three tensor-core passes, which cost nothing here -- the update is latency bound, not MMA bound.
+// Measured against float64 on a B200 (tests/test_td3_kernels_gpu.py): per entry, relative to (|A| |B|)_mn, 1.6-3.0x the
+// FP32 kernel's error on the forward / backward-data products and 5-6x on the split-K backward-weight products (the
+// tensor cores' FP32 accumulation is coarser than round-to-nearest FMA chains), at most 9.6e-7, 2000x below one TF32 pass.
 //
 // One CTA = one 128 x 128 output tile, 512 threads.  K advances in steps of 32 through a two-stage shared-memory ring:
 //   * all threads fetch A (128 x 32) and B (128 x 32) tiles from global memory into registers TWO steps ahead -- arbitrary

@@ -212,9 +212,10 @@ class TD3Agent:                                            # td3.py:196-376
     def __init__(self, state_dim=STATE_DIM, action_dim=ACTION_DIM, max_action=1.0, discount=0.99, tau=0.005,
                  policy_noise=0.2, noise_clip=0.5, policy_freq=2, device="cuda:0", lr=3e-4, max_batch=4096, seed=0,
                  precision="fp32"):
-        """precision: "fp32" = every product on the FP32 CUDA cores, within 1e-5 of torch (the parity path); "tf32" = the
-        products of minibatches >= 128 rows on the tcgen05 tensor cores (TF32 operands, FP32 accumulation; gradients within
-        1e-3 of the fp32 path) -- for minibatches >= 1024, where the update is FLOP bound."""
+        """precision: "fp32" = every product on the FP32 CUDA cores, within 1e-5 of torch (the parity path); "tf32" = for
+        minibatches >= 512 rows, the products that fill a 128-row tile run on the tcgen05 tensor cores (3xTF32: operands
+        split into two TF32 parts, FP32 accumulation; fp32-level accuracy) -- for minibatches >= 1024, where the update is
+        FLOP bound.  Smaller minibatches stay on the FP32 CUDA cores in either precision."""
         if precision not in ("fp32", "tf32"):
             raise ValueError("precision must be 'fp32' or 'tf32'")
         self.precision = precision

@@ -64,3 +64,15 @@ def test_agent_host_logic_without_a_gpu(tmp_path):
     assert torch.equal(b._flat["actor_target"], a._flat["actor"]) and torch.equal(b._flat["critic_target"], a._flat["critic"])
     with pytest.raises(RuntimeError):
         a.train(None, batch=(torch.zeros(4, 26), torch.zeros(4, 18), torch.zeros(4, 26), torch.zeros(4, 1), torch.ones(4, 1)))
+
+
+def test_td3_gemm_harness_compiles_and_loads():
+    """tests/cuda/td3_gemm_harness.cu includes the learner's sources: it must keep compiling for sm_100a and load without
+    undefined symbols, or the GPU tests of the learner's GEMM kernels would break unnoticed when those sources change."""
+    import ctypes
+    import pytest
+    import td3_gemm_util
+    if not os.path.exists(td3_gemm_util.nvcc()):
+        pytest.skip("nvcc not available")
+    lib = ctypes.CDLL(td3_gemm_util.build_harness())
+    assert lib.harness_gemm and lib.harness_tc_timed_out
