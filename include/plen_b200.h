@@ -41,6 +41,7 @@ extern "C" {
 #define PLEN_MAX_BOX_POINTS 4  /* box-vs-ground contact points kept per robot and tick (the deepest ones) */
 #define PLEN_MAX_HULL 256      /* convex-hull vertices of a foot collider (plen.urdf feet: 209 each) */
 #define PLEN_BODIES 19         /* rigid bodies of the robot: the torso composite and the body each of the 18 joints moves */
+#define PLEN_MAX_LATENCY_STEPS 2   /* command latency (plen_set_env_latency) <= PLEN_MAX_LATENCY_STEPS * substeps ticks */
 #define PLEN_MAN_WORDS 52      /* per-robot persistent sole manifold (sole_manifold = 1): [foot][point][local xyz | plane xyz] = 48
                                   floats, the two point counts, 2 spare */
 
@@ -164,7 +165,8 @@ int plen_step(plen_ctx *ctx, const float *actions_dev, float *obs_dev, float *re
  * and a stream synchronise.  This is the end-to-end path a PyBullet user would see.
  * Ordering contract: the call runs on the context's PRIVATE streams (the batch is pipelined in ranges).  It first waits
  * (cudaStreamWaitEvent) for the work the last plen_reset / plen_step / plen_set_state / plen_set_manifold / plen_set_env_scales /
- * plen_set_env_mass / plen_tick call queued on its caller stream, so `plen_reset(...); plen_step_host(...)` needs no synchronisation in between; it
+ * plen_set_env_mass / plen_set_env_latency / plen_tick call queued on its caller stream, so `plen_reset(...); plen_step_host(...)`
+ * needs no synchronisation in between; it
  * returns after its own streams have drained, so whatever the caller queues next is ordered after it.  (Work the caller
  * queued on a stream WITHOUT going through this library -- e.g. a torch kernel still writing the state through
  * plen_set_state's source buffer -- is the caller's to order.) */
@@ -212,6 +214,26 @@ int plen_set_env_mass(plen_ctx *ctx, const float *mass_scale_dev, const float *p
 /* The current values into [N,PLEN_BODIES] / [N,4] device buffers (either NULL to skip), stream-ordered.  Returns 1 when
  * plen_set_env_mass was ever called on this context, 0 when not (the buffers then receive 1 and 0), < 0 on error. */
 int plen_get_env_mass(plen_ctx *ctx, float *mass_scale_dev, float *payload_dev, void *stream);
+
+/* Per-env servo command latency (SURVEY.md 8f-3): the delay between sending a command and the servo acting on it.
+ *   ticks_dev   [N] int32  delay d of each robot in physics ticks, 0 <= d <= PLEN_MAX_LATENCY_STEPS * substeps (0 .. 8 ticks,
+ *               0 .. 33 ms at the default 240 Hz and 4 substeps); a value outside is clamped into that range.
+ *   history_dev [N,2,PLEN_NJ]  the raw servo targets (radians) of the robot's last env step ([:,0]) and of the step before
+ *               ([:,1]), relative to its current episode counter (set the state first); for snapshots that must continue
+ *               a run bit for bit.
+ * Tick k (0-based) of env step t applies the raw targets (after agent_to_env) of step t - s, s = ceil(max(d - k, 0) / substeps):
+ * d = 0 is the stock behaviour, d = substeps applies the previous step's command for the whole step.  A command from before
+ * the robot's last reset (explicit or auto) is the reset-pose hold target 0.  Every plen_step / plen_step_host records each
+ * robot's targets once the history exists; plen_tick, plen_debug_dynamics and the reset snapshot settled at plen_create
+ * neither apply nor record it.  NULL leaves a part as it is.  The first call allocates the history (384 bytes per robot;
+ * until then the context holds none) and fills it with each robot's last servo targets, as if that command had been held,
+ * so a robot switched to a delay mid-episode does not jump to 0; later calls only change what they are given.  Delays may
+ * change between any two steps.  Takes effect from the next step. */
+int plen_set_env_latency(plen_ctx *ctx, const int32_t *ticks_dev, const float *history_dev, void *stream);
+/* The current delays [N] and history [N,2,PLEN_NJ] (same order as above) into device buffers (either NULL to skip),
+ * stream-ordered.  Returns 1 when plen_set_env_latency was ever called on this context, 0 when not (the buffers then receive
+ * 0 and each robot's last servo targets), < 0 on error. */
+int plen_get_env_latency(plen_ctx *ctx, int32_t *ticks_dev, float *history_dev, void *stream);
 
 /* Advance every env by n_ticks physics ticks with raw joint targets [N,18] (radians) and no env logic.
  * Replaces move_joints + p.stepSimulation (plen_env.py:746-753, :665-667); used by the parity tests. */

@@ -21,6 +21,7 @@ AUX_WORDS = 29
 MAX_HULL = 256
 MAN_WORDS = 52          # PLEN_MAN_WORDS
 BODIES = 19             # PLEN_BODIES
+MAX_LATENCY_STEPS = 2   # PLEN_MAX_LATENCY_STEPS
 OBS_DIM = 26
 ACT_DIM = 18
 
@@ -93,7 +94,7 @@ def model_to_c(model: PlenModel) -> PlenModelC:
 
 EXPORTS = (
     "plen_version", "plen_default_config", "plen_create", "plen_destroy", "plen_last_error", "plen_num_envs", "plen_kernel_launches",
-    "plen_reset", "plen_step", "plen_step_host", "plen_fault_count", "plen_get_state", "plen_set_state", "plen_set_env_scales", "plen_set_env_mass", "plen_get_env_mass", "plen_get_manifold", "plen_set_manifold", "plen_tick",
+    "plen_reset", "plen_step", "plen_step_host", "plen_fault_count", "plen_get_state", "plen_set_state", "plen_set_env_scales", "plen_set_env_mass", "plen_get_env_mass", "plen_set_env_latency", "plen_get_env_latency", "plen_get_manifold", "plen_set_manifold", "plen_tick",
     "plen_debug_dynamics", "plen_debug_records", "plen_gait_ik", "plen_profile_enable", "plen_profile_read", "plen_measure_fp32_peak",
     "plen_replay_create", "plen_replay_destroy", "plen_replay_size", "plen_replay_ptr", "plen_replay_storage",
     "plen_replay_add", "plen_replay_sample", "plen_actor_forward", "plen_actor_forward_tc", "plen_actor_tc_timed_out", "plen_td3_last_error", "plen_td3_set_precision", "plen_td3_tc_timed_out",
@@ -149,6 +150,8 @@ def load_library(path: str = LIB_PATH):
     L.plen_set_env_scales.argtypes = [vp] * 5
     L.plen_set_env_mass.argtypes = [vp] * 4
     L.plen_get_env_mass.argtypes = [vp] * 4
+    L.plen_set_env_latency.argtypes = [vp] * 4
+    L.plen_get_env_latency.argtypes = [vp] * 4
     L.plen_tick.argtypes = [vp, vp, ip, vp]
     L.plen_get_manifold.argtypes = [vp, vp, vp]
     L.plen_set_manifold.argtypes = [vp, vp, vp]

@@ -54,8 +54,10 @@ struct plen_ctx {
     float *d_tgt;    // [n][18] servo targets of the current env step
     float *d_man;    // [n][PLEN_MAN_WORDS] persistent sole manifolds (cfg.sole_manifold = 1; NULL otherwise)
     float *d_hull;   // [2][PLEN_MAX_HULL][3] hull vertices of the feet (ditto)
-    float *d_scale;  // [n][4] per-robot scales: friction, servo force limit, servo gain, reserved (plen_set_env_scales; all 1)
+    float *d_scale;  // [n][4] per-robot scales: friction, servo force limit, servo gain (plen_set_env_scales; all 1), and the
+                     // command delay in ticks (word SC_LATENCY, plen_set_env_latency; read only while d_lat exists)
     float *d_mass;   // [n][MR_WORDS] per-robot body mass scales and torso payload (plen_set_env_mass; NULL until its first call)
+    float *d_lat;    // [n][LAT_WORDS] per-robot command history ring (plen_set_env_latency; NULL until its first call)
     uint8_t *d_key;  // [n] contact-load sort key of the current tick (k_dyn -> k_rank)
     int *d_perm;     // [n_tiles * RANK_TILE] robots ordered by contact load inside each tile (k_rank -> k_solve)
     float *d_act, *d_obs, *d_rew;
@@ -109,12 +111,15 @@ __device__ __forceinline__ DynSmem &stage_table(const float *tab_g) {
 // 5 CTAs (20 warps) per SM: the register cap (<= 102) costs 16 B of spills outside the hot loops and measured +2.4 %
 // MASS = true: the robots' mass rows (mrow, [n][MR_WORDS]) scale their bodies and add the torso payload; the false instance is
 // the stock path, untouched by the option (launched whenever no mass row applies).
+// lat != NULL (env steps once plen_set_env_latency was called; then scale != NULL too): tick `tick` of the step applies the
+// robot's delayed command (latency_source) from its history ring, and tick 0 records the step's own targets in the ring.
 template <bool MASS>
 __global__ void __launch_bounds__(DYN_WPC * 32, DYN_CTAS)
 k_dyn(const __grid_constant__ DevConfig dc, const __grid_constant__ EnvRanges er, const float *__restrict__ tab_g,
       const float *__restrict__ state, int n, const float *__restrict__ actions, float *__restrict__ tgt,
       float *__restrict__ srec, uint8_t *__restrict__ keys, float *dbg_minv, float *dbg_pos, float *dbg_rot,
-      const float *__restrict__ scale, float *__restrict__ srx, float *__restrict__ man, const float *__restrict__ mrow) {
+      const float *__restrict__ scale, float *__restrict__ srx, float *__restrict__ man, const float *__restrict__ mrow,
+      float *__restrict__ lat, int tick) {
     // The 4 KB model table is staged with cp.async while every warp already fetches its robot's state record and targets:
     // the two latencies overlap instead of adding up (the table wait used to sit in front of everything).
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -138,6 +143,13 @@ k_dyn(const __grid_constant__ DevConfig dc, const __grid_constant__ EnvRanges er
     if (has && scale) sc = gld4(scale + 4 * (size_t)env);
     float mw = 1.0f;
     if (MASS && has) mw = gld(mrow + (size_t)env * MR_WORDS + lane);     // one 128-byte line per robot
+    int lsrc = 0, ept = 0;
+    float lv = 0.0f;       // the delayed targets (0: the reset-pose hold target of a command from before the last reset)
+    if (lat && has) {
+        ept = max((int)shfl(r1, W_EPT - 32), 0);
+        lsrc = latency_source((int)sc.w, tick, dc.substeps, ept);
+        if (lsrc > 0 && jl) lv = gld(lat + (size_t)env * LAT_WORDS + 32 * latency_slot(ept, lsrc) + lane);   // one ring row
+    }
     asm volatile("cp.async.wait_all;" ::: "memory");
     __syncthreads();
     if (!has) return;
@@ -148,6 +160,10 @@ k_dyn(const __grid_constant__ DevConfig dc, const __grid_constant__ EnvRanges er
     if (jl) {
         if (actions) { L.tgt = agent_target(dc, er, lane - 6, a_in); tgt[o] = L.tgt; }
         else L.tgt = a_in;
+        if (lat) {
+            if (actions) lat[(size_t)env * LAT_WORDS + 32 * latency_slot(ept, 0) + lane] = L.tgt;   // this step joins the history
+            if (lsrc != 0) L.tgt = lv;
+        }
     }
     DebugOut dbg{dbg_minv ? dbg_minv + (size_t)env * 576 : nullptr, dbg_pos ? dbg_pos + (size_t)env * 72 : nullptr,
                  dbg_rot ? dbg_rot + (size_t)env * 216 : nullptr};
@@ -301,6 +317,43 @@ __global__ void k_get_mass(const float *__restrict__ mrow, int n, float *scale, 
     const bool pay = w >= MR_PAYLOAD && w < MR_PAYLOAD + 4, body = w == 0 || (w >= 6 && w < MR_PAYLOAD);
     if (scale && body) scale[e * PLEN_BODIES + (w == 0 ? 0 : w - 5)] = mrow ? mrow[i] : 1.0f;
     if (payload && pay) payload[e * 4 + (w - MR_PAYLOAD)] = mrow ? mrow[i] : 0.0f;
+}
+
+// per-robot command latency, one thread per robot: the delay (clamped to 0 .. 2 substeps, so that no value can index out of
+// the ring) into word SC_LATENCY of the scale row, the logical history [n][2][18] (last step, the step before) into the ring
+// rows of the robot's episode counter.  NULL leaves a part as it is; `init` first sets delay 0 and fills every ring row with
+// the robot's last targets (tgt), as if that command had been held.
+__global__ void k_set_latency(float *__restrict__ scale, float *__restrict__ ring, const float *__restrict__ state,
+                              const float *__restrict__ tgt, int n, int max_ticks, const int *ticks, const float *hist, int init) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    float *row = ring + (size_t)e * LAT_WORDS;
+    if (init) {
+        scale[4 * (size_t)e + SC_LATENCY] = 0.0f;
+        for (int s = 0; s < LAT_SLOTS; s++)
+            for (int j = 0; j < PLEN_NJ; j++) row[32 * s + 6 + j] = tgt[(size_t)e * PLEN_NJ + j];
+    }
+    if (ticks) scale[4 * (size_t)e + SC_LATENCY] = (float)min(max(ticks[e], 0), max_ticks);
+    if (hist) {
+        const int ept = max((int)state[(size_t)e * PLEN_STATE_WORDS + W_EPT], 0);
+        for (int s = 1; s <= 2; s++)
+            for (int j = 0; j < PLEN_NJ; j++) row[32 * latency_slot(ept, s) + 6 + j] = hist[((size_t)e * 2 + s - 1) * PLEN_NJ + j];
+    }
+}
+
+// ... and back; delay 0 and the last targets as history when the context has no ring
+__global__ void k_get_latency(const float *__restrict__ scale, const float *__restrict__ ring, const float *__restrict__ state,
+                              const float *__restrict__ tgt, int n, int *ticks, float *hist) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    if (ticks) ticks[e] = ring ? (int)scale[4 * (size_t)e + SC_LATENCY] : 0;
+    if (hist) {
+        const int ept = max((int)state[(size_t)e * PLEN_STATE_WORDS + W_EPT], 0);
+        for (int s = 1; s <= 2; s++)
+            for (int j = 0; j < PLEN_NJ; j++)
+                hist[((size_t)e * 2 + s - 1) * PLEN_NJ + j] =
+                    ring ? ring[(size_t)e * LAT_WORDS + 32 * latency_slot(ept, s) + 6 + j] : tgt[(size_t)e * PLEN_NJ + j];
+    }
 }
 
 // After the last tick of an env step, one warp per robot: observation, done, reward, counters, auto-reset.
@@ -551,16 +604,17 @@ static const size_t SOLVE_X_SMEM = sizeof(float) * (PLEN_GS_WORDS + PLEN_XS_WORD
 static int dyn_grid(int n) { return (n + DYN_WPC - 1) / DYN_WPC; }
 static int rank_tiles(int n) { return (n + RANK_TILE - 1) / RANK_TILE; }
 
-// k_dyn over n robots; the MASS instance only when mass rows apply (mrow != NULL), the stock instance otherwise
+// k_dyn over n robots; the MASS instance only when mass rows apply (mrow != NULL), the stock instance otherwise.  lat: the
+// robots' command history rings (nullable), tick: index of the tick inside the env step
 static void launch_dyn(plen_ctx *ctx, const float *state, int n, const float *actions, float *tgt, float *srec, uint8_t *key,
                        float *dbg_minv, float *dbg_pos, float *dbg_rot, const float *scale, float *srx, float *man,
-                       const float *mrow, cudaStream_t st) {
+                       const float *mrow, float *lat, int tick, cudaStream_t st) {
     if (mrow)
         k_dyn<true><<<dyn_grid(n), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->dc, ctx->er, ctx->d_tab, state, n, actions, tgt, srec, key,
-                                                                dbg_minv, dbg_pos, dbg_rot, scale, srx, man, mrow);
+                                                                dbg_minv, dbg_pos, dbg_rot, scale, srx, man, mrow, lat, tick);
     else
         k_dyn<false><<<dyn_grid(n), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->dc, ctx->er, ctx->d_tab, state, n, actions, tgt, srec, key,
-                                                                 dbg_minv, dbg_pos, dbg_rot, scale, srx, man, nullptr);
+                                                                 dbg_minv, dbg_pos, dbg_rot, scale, srx, man, nullptr, lat, tick);
 }
 
 // n_ticks physics ticks of 1/240 s: (k_dyn, k_solve) per tick.  `actions` (agent space) only on the first tick.
@@ -581,9 +635,11 @@ static void launch_ticks(plen_ctx *ctx, float *state, int n, const float *action
     const bool snap = state == ctx->d_snapshot;
     const float *scale = (snap || !ctx->d_scale) ? nullptr : ctx->d_scale + 4 * off;
     const float *mrow = (snap || !ctx->d_mass) ? nullptr : ctx->d_mass + MR_WORDS * off;
+    // command latency: env steps only (agent actions); plen_tick and the snapshot settle run raw physics without it
+    float *lat = (snap || !actions || !ctx->d_lat) ? nullptr : ctx->d_lat + LAT_WORDS * off;
     for (int t = 0; t < n_ticks; t++) {
         if (ev) cudaEventRecord(ev[2 * t], st);
-        launch_dyn(ctx, state, n, t == 0 ? actions : nullptr, tgt, srec, key, nullptr, nullptr, nullptr, scale, srx, man, mrow, st);
+        launch_dyn(ctx, state, n, t == 0 ? actions : nullptr, tgt, srec, key, nullptr, nullptr, nullptr, scale, srx, man, mrow, lat, t, st);
         if (ev) cudaEventRecord(ev[2 * t + 1], st);
         const int nt = rank_tiles(n);
         k_rank<<<nt, RANK_TILE, 0, st>>>(key, n, perm, xg);
@@ -643,7 +699,7 @@ unsigned long long plen_kernel_launches(const plen_ctx *ctx) { return ctx ? ctx-
 void plen_destroy(plen_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    cudaFree(ctx->d_tab); cudaFree(ctx->d_state); cudaFree(ctx->d_snapshot); cudaFree(ctx->d_srec); cudaFree(ctx->d_srx); cudaFree(ctx->d_xgroups); cudaFree(ctx->d_tgt); cudaFree(ctx->d_key); cudaFree(ctx->d_perm); cudaFree(ctx->d_scale); cudaFree(ctx->d_mass); cudaFree(ctx->d_man); cudaFree(ctx->d_hull);
+    cudaFree(ctx->d_tab); cudaFree(ctx->d_state); cudaFree(ctx->d_snapshot); cudaFree(ctx->d_srec); cudaFree(ctx->d_srx); cudaFree(ctx->d_xgroups); cudaFree(ctx->d_tgt); cudaFree(ctx->d_key); cudaFree(ctx->d_perm); cudaFree(ctx->d_scale); cudaFree(ctx->d_mass); cudaFree(ctx->d_lat); cudaFree(ctx->d_man); cudaFree(ctx->d_hull);
     cudaFree(ctx->d_act); cudaFree(ctx->d_obs); cudaFree(ctx->d_rew); cudaFree(ctx->d_done); cudaFree(ctx->d_tmo); cudaFree(ctx->d_faults);
     for (int k = 1; k < PLEN_HOST_PIPE; k++)
         if (ctx->pipe[k]) cudaStreamDestroy(ctx->pipe[k]);
@@ -711,6 +767,8 @@ static int create_impl(plen_ctx *ctx) {
         CK(ctx, cudaMalloc(&ctx->d_xgroups, sizeof(int) * ((size_t)rank_tiles(n) + 1)));
     }
     CK(ctx, cudaMalloc(&ctx->d_tgt, sizeof(float) * PLEN_NJ * (size_t)n));
+    // the reset-pose hold target until the first step: plen_set_env_latency seeds the command history from these
+    CK(ctx, cudaMemset(ctx->d_tgt, 0, sizeof(float) * PLEN_NJ * (size_t)n));
     CK(ctx, cudaMalloc(&ctx->d_key, (size_t)n));
     CK(ctx, cudaMalloc(&ctx->d_perm, sizeof(int) * (size_t)rank_tiles(n) * RANK_TILE));
     CK(ctx, cudaMalloc(&ctx->d_scale, sizeof(float) * 4 * (size_t)n));
@@ -855,8 +913,8 @@ int plen_step_host(plen_ctx *ctx, const float *actions_host, float *obs_host, fl
         const size_t off = bound[used], cnt = bound[used + 1] - off;
         cudaStream_t st = ctx->pipe[used % PLEN_HOST_PIPE];
         // ordering contract (plen_b200.h): this call runs on the context's private streams, so it first waits for whatever
-        // the last stream-taking entry point (reset / step / set_state / set_env_scales / set_env_mass / tick) queued on the
-        // caller's stream
+        // the last stream-taking entry point (reset / step / set_state / set_env_scales / set_env_mass / set_env_latency /
+        // tick) queued on the caller's stream
         CK(ctx, cudaStreamWaitEvent(st, ctx->last_work, 0));
         CK(ctx, cudaMemcpyAsync(ctx->d_act + off * PLEN_NJ, actions_host + off * PLEN_NJ, sizeof(float) * PLEN_NJ * cnt,
                                 cudaMemcpyHostToDevice, st));
@@ -902,6 +960,38 @@ int plen_get_env_mass(plen_ctx *ctx, float *mass_scale_dev, float *payload_dev, 
     k_get_mass<<<(unsigned)((words + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ctx->d_mass, ctx->n, mass_scale_dev, payload_dev);
     CK(ctx, cudaGetLastError());
     return ctx->d_mass ? 1 : 0;
+}
+
+int plen_set_env_latency(plen_ctx *ctx, const int32_t *ticks_dev, const float *history_dev, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    CK(ctx, cudaSetDevice(ctx->device));
+    const int init = !ctx->d_lat;           // the ring is allocated at the first call: a context that never sets it has none
+    if (init) {
+        cudaError_t e = cudaMalloc(&ctx->d_lat, sizeof(float) * LAT_WORDS * (size_t)ctx->n);
+        if (e != cudaSuccess) {
+            ctx->d_lat = nullptr;
+            return fail(ctx, PLEN_E_CUDA, "plen_set_env_latency: cudaMalloc: %s", cudaGetErrorString(e));
+        }
+    }
+    k_set_latency<<<(ctx->n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ctx->d_scale, ctx->d_lat, ctx->d_state, ctx->d_tgt, ctx->n,
+                                                                        PLEN_MAX_LATENCY_STEPS * ctx->cfg.substeps, ticks_dev,
+                                                                        history_dev, init);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        if (init) { cudaFree(ctx->d_lat); ctx->d_lat = nullptr; }    // an unseeded ring must never be stepped with
+        return fail(ctx, PLEN_E_CUDA, "plen_set_env_latency: k_set_latency: %s", cudaGetErrorString(e));
+    }
+    CK(ctx, mark_work(ctx, (cudaStream_t)stream));
+    return PLEN_OK;
+}
+
+int plen_get_env_latency(plen_ctx *ctx, int32_t *ticks_dev, float *history_dev, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    CK(ctx, cudaSetDevice(ctx->device));
+    k_get_latency<<<(ctx->n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ctx->d_scale, ctx->d_lat, ctx->d_state, ctx->d_tgt, ctx->n,
+                                                                        ticks_dev, history_dev);
+    CK(ctx, cudaGetLastError());
+    return ctx->d_lat ? 1 : 0;
 }
 
 int plen_get_manifold(plen_ctx *ctx, float *man_dev, void *stream) {
@@ -963,7 +1053,7 @@ int plen_debug_dynamics(plen_ctx *ctx, float *minv_dev, float *pos_dev, float *r
     if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
     launch_dyn(ctx, ctx->d_state, ctx->n, nullptr, nullptr, ctx->d_srec, ctx->d_key, minv_dev, pos_dev, rot_dev, ctx->d_scale, ctx->d_srx,
-               nullptr /* diagnostics must not advance the manifolds */, ctx->d_mass, (cudaStream_t)stream);
+               nullptr /* diagnostics must not advance the manifolds */, ctx->d_mass, nullptr, 0, (cudaStream_t)stream);
     CK(ctx, cudaGetLastError());
     return PLEN_OK;
 }

@@ -246,6 +246,13 @@ struct LaneState {
 // per-robot mass row (plen_set_env_mass): 32 words, one per lane, so that a warp reads it with one 128-byte load
 enum { MR_PAYLOAD = 24, MR_WORDS = 32 };
 
+// per-robot command latency (plen_set_env_latency): the delay d in ticks is word SC_LATENCY of the robot's scale row (d_scale,
+// [n][4], loaded by k_dyn anyway; plen_set_env_scales never writes that word), kept as a float holding an integer.  The
+// command history is a ring of LAT_SLOTS 128-byte rows per robot ([n][LAT_WORDS]): the raw servo targets of the step whose
+// episode counter is e sit in row e mod LAT_SLOTS, lanes 6..23 (the other lanes are unused).  Tick 0 of a step writes its
+// row while the rows of the two steps before stay readable, so no row is ever copied.
+enum { SC_LATENCY = 3, LAT_SLOTS = 3, LAT_WORDS = LAT_SLOTS * 32 };
+
 PLEN_DEV void mat3_mul(const float *A, const float *B, float *C) {
 #pragma unroll
     for (int i = 0; i < 3; i++)

@@ -107,6 +107,18 @@ PLEN_DEV float agent_target(const DevConfig &cfg, const EnvRanges &rng, int j, f
     return (float)y;
 }
 
+// Per-robot command latency (plen_set_env_latency): tick k (0 <= k < S = substeps) of an env step applies the raw targets
+// of the step s = ceil(max(d - k, 0) / S) steps back, s = 0, 1 or 2 for a delay of 0 <= d <= 2 S ticks.  ep_t is the
+// robot's episode counter (steps since its last reset) at this step; a command from before that reset is the reset-pose
+// hold target 0, returned as -1.
+PLEN_DEV int latency_source(int d, int k, int S, int ep_t) {
+    const int late = d - k;
+    const int s = late > 0 ? (late + S - 1) / S : 0;
+    return (s == 0 || s <= ep_t) ? s : -1;
+}
+// ring row (LAT_SLOTS rows per robot) of the targets s steps before the step with episode counter ep_t (0 <= s <= 2, ep_t >= 0)
+PLEN_DEV int latency_slot(int ep_t, int s) { return (ep_t + LAT_SLOTS - s) % LAT_SLOTS; }
+
 // Everything of PlenWalkEnv.step after the 4 physics ticks (:671-678) + TimeLimit + optional auto-reset (k_post).
 PLEN_DEV void env_post(const DevConfig &cfg, const float *tab, WarpScratch &ws, LaneState &L, int lane,
                        const StepIO &io) {

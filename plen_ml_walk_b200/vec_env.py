@@ -274,14 +274,67 @@ class PlenVecEnv:
         s, p, _ = self._get_env_mass()
         return s, p
 
+    @property
+    def max_latency_ticks(self):
+        """Largest command delay set_env_latency accepts: 2 * substeps physics ticks (8 ticks, 33 ms at the defaults)."""
+        return _abi.MAX_LATENCY_STEPS * int(self.cfg.substeps)
+
+    def set_env_latency(self, ticks, history=None):
+        """Per-env servo command latency (SURVEY.md 8f-3): each robot's servos act on its commands `ticks` physics ticks late.
+
+        ticks:   an int (every robot) or [N] integers, 0 <= d <= max_latency_ticks; one tick is 1/240 s = 4.17 ms at the default
+                 rate.  Tick k of a step (0 <= k < substeps) applies the raw servo targets of the step ceil(max(d - k, 0) /
+                 substeps) steps back: 0 is the stock behaviour, d = substeps applies the previous step's command for the
+                 whole step.  A command from before the robot's last reset (explicit or auto-reset) is the reset-pose hold
+                 target 0 rad.
+        history: [N,2,18] raw targets of the last step and of the step before (radians, relative to the robots' current
+                 episode counters), None to keep the recorded ones; load_state uses it to continue a run bit for bit.
+        Raises ValueError on a wrong shape, a non-integer, a negative value or a value above max_latency_ticks.
+        The first call starts a command history seeded with each robot's last servo targets, as if they had been held;
+        every step() / step_host() records into it from then on.  Delays may change between any two steps.  tick() and
+        debug_dynamics() are raw physics and ignore the latency."""
+        n = self.num_envs
+        t = torch.as_tensor(ticks, device=self.device)
+        if t.dim() == 0:
+            t = t.expand(n)
+        if tuple(t.shape) != (n,):
+            raise ValueError("ticks: expected an int or shape (%d,), got %s" % (n, tuple(t.shape)))
+        if t.dtype.is_floating_point:
+            if not bool(torch.isfinite(t).all()) or not bool((t == torch.round(t)).all()):
+                raise ValueError("ticks must be integers")
+        elif t.dtype == torch.bool or t.dtype.is_complex:
+            raise ValueError("ticks must be integers")
+        if not bool((t >= 0).all()) or not bool((t <= self.max_latency_ticks).all()):
+            raise ValueError("ticks must lie in 0 .. %d (2 * substeps)" % self.max_latency_ticks)
+        t = t.to(torch.int32).contiguous()
+        h = None if history is None else self._dev_f32(history, (n, 2, ACT_DIM))
+        with torch.cuda.device(self.device):
+            self._check(self.lib.plen_set_env_latency(self._ctx, self._p(t), self._p(h), self._stream()))
+
+    def _get_env_latency(self):
+        n, dev = self.num_envs, self.device
+        t = torch.empty(n, dtype=torch.int32, device=dev)
+        h = torch.empty((n, 2, ACT_DIM), dtype=torch.float32, device=dev)
+        with torch.cuda.device(self.device):
+            rc = self.lib.plen_get_env_latency(self._ctx, self._p(t), self._p(h), self._stream())
+        if rc < 0:
+            self._check(rc)
+        return t, h, rc == 1
+
+    def get_env_latency(self):
+        """-> int32 [N]: each robot's command delay in physics ticks (0 where set_env_latency was never called)."""
+        return self._get_env_latency()[0]
+
     def save_state(self, path):
-        """Snapshot of every env (pose, velocities, contact cache, env bookkeeping, per-env scales and masses) to one .pt file
-        (SURVEY.md 8f-4)."""
+        """Snapshot of every env (pose, velocities, contact cache, env bookkeeping, per-env scales, masses, command delays and
+        command history) to one .pt file (SURVEY.md 8f-4)."""
         qpos, qvel, aux = self.get_state()
         ms, mp, mass_set = self._get_env_mass()
+        lt, lh, lat_set = self._get_env_latency()
         torch.save({"num_envs": self.num_envs, "joint_act": self.joint_act, "qpos": qpos.cpu(), "qvel": qvel.cpu(), "aux": aux.cpu(),
                     "scales": {k: v.cpu() for k, v in self._scales.items()},
                     "mass": {"scale": ms.cpu(), "payload": mp.cpu()} if mass_set else None,
+                    "latency": {"ticks": lt.cpu(), "history": lh.cpu()} if lat_set else None,
                     "manifold": self.get_manifold().cpu() if int(self.cfg.sole_manifold) else None}, path)
 
     def load_state(self, path):
@@ -301,6 +354,11 @@ class PlenVecEnv:
             self.set_env_mass(mass["scale"], mass["payload"])
         elif self._get_env_mass()[2]:
             self.set_env_mass(torch.ones(self.num_envs, _abi.BODIES), torch.zeros(self.num_envs, 4))
+        lat = d.get("latency")
+        if lat is not None:         # after set_state: the history is written relative to the restored episode counters
+            self.set_env_latency(lat["ticks"], lat["history"])
+        elif self._get_env_latency()[2]:
+            self.set_env_latency(0)
 
     def tick(self, targets, n_ticks=1):
         """Raw physics: n_ticks of 1/240 s with joint targets in radians, no env logic (move_joints + stepSimulation)."""

@@ -9,10 +9,12 @@ rollout (reset and policy are deterministic, so every noise-free env is identica
 noise to give a distribution.  Reports episode length / return of the first episode and the distance walked.
 
     python scripts/walk_eval_batched.py [--envs 4096] [--sigma 0.05] [--precision fp32|fp16]
-                                        [--mass-scale S] [--payload KG [--payload-offset X Y Z]]
+                                        [--mass-scale S] [--payload KG [--payload-offset X Y Z]] [--latency-ticks D | LO:HI]
 
 --mass-scale / --payload sweep the policy's robustness to the robot's mass (PlenVecEnv.set_env_mass): every body x S, and a
-point mass of KG kg on the torso, by default at the torso body's centre of mass.
+point mass of KG kg on the torso, by default at the torso body's centre of mass.  --latency-ticks sweeps its robustness to servo
+command latency (PlenVecEnv.set_env_latency): every robot's servos act D physics ticks (4.17 ms each at 240 Hz) late, or a
+delay drawn uniformly from LO..HI per robot (seeded).
 """
 import argparse
 import json
@@ -43,6 +45,8 @@ def main():
     ap.add_argument("--payload", type=float, default=None, metavar="KG", help="point mass on the torso, kg")
     ap.add_argument("--payload-offset", type=float, nargs=3, default=None, metavar=("X", "Y", "Z"),
                     help="where the payload sits in the torso body frame, m (default: the torso's centre of mass)")
+    ap.add_argument("--latency-ticks", default=None, metavar="D|LO:HI",
+                    help="servo command latency in physics ticks (0 .. 2 * substeps), or LO:HI for a uniform draw per robot")
     a = ap.parse_args()
     dev = torch.device("cuda:0")
     g = np.load(GOLD)
@@ -60,6 +64,13 @@ def main():
         pay = torch.tensor([a.payload or 0.0] + at, dtype=torch.float32).expand(n, 4)
         env.set_env_mass(None if a.mass_scale is None else torch.full((n,), a.mass_scale), pay if a.payload is not None else None)
         mass = {"mass_scale": a.mass_scale, "payload_kg": a.payload, "payload_at_m": at if a.payload is not None else None}
+    latency = None
+    if a.latency_ticks is not None:
+        lo, _, hi = a.latency_ticks.partition(":")
+        lo, hi = int(lo), int(hi or lo)
+        gen = torch.Generator(device=dev); gen.manual_seed(0)
+        env.set_env_latency(torch.randint(lo, hi + 1, (n,), device=dev, generator=gen))
+        latency = {"ticks_lo": lo, "ticks_hi": hi, "ms_per_tick": 1000.0 * float(env.cfg.dt)}
     state = env.reset().clone()
     alive = torch.ones(n, dtype=torch.bool, device=dev)
     ep_len = torch.zeros(n, device=dev); ep_ret = torch.zeros(n, device=dev)
@@ -78,7 +89,7 @@ def main():
     L, R, X = ep_len.cpu().numpy(), ep_ret.cpu().numpy(), x_end.cpu().numpy()
     print(json.dumps({
         "policy": "plen_walk_gazebo_3229999 (reference checkpoint)", "envs": n, "steps": a.steps, "sigma": a.sigma,
-        "precision": a.precision, "sole_manifold": a.sole_manifold, "config_overrides": ovr, "mass": mass,
+        "precision": a.precision, "sole_manifold": a.sole_manifold, "config_overrides": ovr, "mass": mass, "latency": latency,
         "deterministic": {"episode_length": float(L[0]), "return": float(R[0]), "x_final_m": float(X[0])},
         "noisy": {"episode_length_mean": float(L[1:].mean()), "episode_length_median": float(np.median(L[1:])),
                   "survived_all_steps_frac": float((L[1:] >= a.steps).mean()), "return_mean": float(R[1:].mean()),
