@@ -141,11 +141,13 @@ plen_ctx *plen_create(const plen_config *cfg, const plen_model *model, int n_env
 void plen_destroy(plen_ctx *ctx);
 const char *plen_last_error(const plen_ctx *ctx);
 int plen_num_envs(const plen_ctx *ctx);
-/* Kernels launched so far by plen_reset / plen_step / plen_step_host / plen_tick on this context (13 per step and range:
- * plen_step_host runs up to four ranges, plen_step of 2,048 robots or more runs two); bench.py's gpu_launches reads it. */
+/* Kernels launched so far by plen_reset / plen_step / plen_step_host / plen_tick / plen_settle_env_resets on this context (13
+ * per step and range: plen_step_host runs up to four ranges, plen_step of 2,048 robots or more runs two; a settle launches its
+ * reset_ticks ticks over the whole batch plus 2); bench.py's gpu_launches reads it. */
 unsigned long long plen_kernel_launches(const plen_ctx *ctx);
 
-/* Replaces PlenWalkEnv.reset (plen_env.py:558-614) for the envs whose mask byte is non-zero (NULL = all).
+/* Replaces PlenWalkEnv.reset (plen_env.py:558-614) for the envs whose mask byte is non-zero (NULL = all): each restores the
+ * post-reset snapshot, or its own row of the reset table once plen_settle_env_resets / plen_set_env_resets made one.
  * obs_dev may be NULL. */
 int plen_reset(plen_ctx *ctx, const uint8_t *mask_dev, float *obs_dev, void *stream);
 
@@ -165,7 +167,8 @@ int plen_step(plen_ctx *ctx, const float *actions_dev, float *obs_dev, float *re
  * and a stream synchronise.  This is the end-to-end path a PyBullet user would see.
  * Ordering contract: the call runs on the context's PRIVATE streams (the batch is pipelined in ranges).  It first waits
  * (cudaStreamWaitEvent) for the work the last plen_reset / plen_step / plen_set_state / plen_set_manifold / plen_set_env_scales /
- * plen_set_env_mass / plen_set_env_latency / plen_tick call queued on its caller stream, so `plen_reset(...); plen_step_host(...)`
+ * plen_set_env_mass / plen_set_env_latency / plen_settle_env_resets / plen_set_env_resets / plen_clear_env_resets / plen_tick call
+ * queued on its caller stream, so `plen_reset(...); plen_step_host(...)`
  * needs no synchronisation in between; it
  * returns after its own streams have drained, so whatever the caller queues next is ordered after it.  (Work the caller
  * queued on a stream WITHOUT going through this library -- e.g. a torch kernel still writing the state through
@@ -194,7 +197,10 @@ int plen_set_manifold(plen_ctx *ctx, const float *man_dev, void *stream);
 /* Per-env domain randomisation (the reference lists it as future work, README.md:75-76; SURVEY.md 8f-3): scale factors of
  * the three foot friction coefficients (plen_env.py:309, 439-452), of the servo force limit (setJointMotorControlArray
  * forces=0.15, plen_env.py:753) and of the servo position gain (POSITION_CONTROL kp 0.1).  Arrays are [N] device floats;
- * NULL leaves a column as it is; every scale is 1 after plen_create.  Takes effect from the next tick. */
+ * NULL leaves a column as it is; every scale is 1 after plen_create.  Takes effect from the next tick.
+ * Resets: a reset (explicit or auto) restores the ONE snapshot settled under unit scales at plen_create, whatever the robot's
+ * own scales are -- unless plen_settle_env_resets has settled each robot's reset state under its own scales (call it after
+ * the setters). */
 int plen_set_env_scales(plen_ctx *ctx, const float *friction_scale_dev, const float *motor_force_scale_dev,
                         const float *motor_gain_scale_dev, void *stream);
 
@@ -208,8 +214,9 @@ int plen_set_env_scales(plen_ctx *ctx, const float *friction_scale_dev, const fl
  * table at all (the first call allocates 128 bytes per robot); a robot with scale 1 and payload 0 steps bit-identically to a
  * context that never called this.  Takes effect from the next tick.  Precondition: scales finite and > 0, m finite and >= 0,
  * x y z finite; a violation produces non-finite states, which the numeric guard retires (plen_fault_count).
- * Approximation, as for plen_set_env_scales: a reset (explicit or auto) restores the ONE snapshot settled under the nominal
- * model at plen_create; the robot's own masses apply from its first tick after that. */
+ * Resets: as for plen_set_env_scales, a reset (explicit or auto) restores the ONE snapshot settled under the nominal model at
+ * plen_create, and the robot's own masses apply from its first tick after that -- unless plen_settle_env_resets has settled
+ * each robot's reset state under its own parameters. */
 int plen_set_env_mass(plen_ctx *ctx, const float *mass_scale_dev, const float *payload_dev, void *stream);
 /* The current values into [N,PLEN_BODIES] / [N,4] device buffers (either NULL to skip), stream-ordered.  Returns 1 when
  * plen_set_env_mass was ever called on this context, 0 when not (the buffers then receive 1 and 0), < 0 on error. */
@@ -234,6 +241,38 @@ int plen_set_env_latency(plen_ctx *ctx, const int32_t *ticks_dev, const float *h
  * stream-ordered.  Returns 1 when plen_set_env_latency was ever called on this context, 0 when not (the buffers then receive
  * 0 and each robot's last servo targets), < 0 on error. */
 int plen_get_env_latency(plen_ctx *ctx, int32_t *ticks_dev, float *history_dev, void *stream);
+
+/* Per-env reset states (no reference counterpart: the reference resets every robot to one pose, plen_env.py:558-574).
+ * A context starts without a reset table: every reset restores the one snapshot settled at plen_create.  The first
+ * plen_settle_env_resets or plen_set_env_resets call allocates one row per robot (720 bytes, plus 592 bytes of settle scratch),
+ * filled with that snapshot; from then on every reset of robot e -- plen_reset, the auto-reset of plen_step / plen_step_host and
+ * the numeric guard, including the terminal observation of a faulted robot -- restores row e: record, observation and sole
+ * manifolds.  The running states are never touched by these calls; a new row applies from the robot's next reset.
+ *
+ * plen_settle_env_resets runs the reference's reset procedure for every robot under its CURRENT friction, force and gain
+ * scales and mass rows: the robot at its start pose with joints, velocities, targets and contact cache zero and empty sole
+ * manifolds, then config.reset_ticks ticks with hold target 0; the result becomes its row.
+ *   start_dev [N,4] (x, y, z, yaw): base position in the world and heading about world z, quaternion (0, 0, sin(yaw/2),
+ *             cos(yaw/2)); NULL = config.start_pos and yaw 0 for every robot (a nominal robot's row is then the snapshot bit
+ *             for bit).  Precondition: finite values; a non-finite pose settles into a non-finite row, which the numeric
+ *             guard retires at the robot's first step after a reset.
+ * Command latency does not apply (the settle, like plen_tick and the snapshot settle, is raw physics); the command history
+ * and its rule that a command from before the last reset is the hold target 0 stay as they are.  Call it after the setters
+ * whose parameters the rows should reflect.  Launches reset_ticks physics ticks over the whole batch plus 2 kernels.
+ *
+ * plen_set_env_resets: user-supplied reset states in the layouts of plen_set_state (qpos [N,25], qvel [N,24],
+ * aux [N,PLEN_AUX_WORDS]) and plen_set_manifold (man [N,PLEN_MAN_WORDS]; PLEN_E_STATE when config.sole_manifold = 0); NULL
+ * leaves that part of every row as it is.  Each row's observation is computed from its record.
+ * plen_get_env_resets: the rows into device buffers of the same layouts plus obs [N,26]; any pointer may be NULL (man needs
+ * sole_manifold = 1, as above).  Returns 1 when the context has a table, 0 when not (every robot then receives the shared
+ * snapshot), < 0 on error.
+ * plen_clear_env_resets: synchronises `stream` and frees the table; the context is then exactly the stock path again. */
+int plen_settle_env_resets(plen_ctx *ctx, const float *start_dev, void *stream);
+int plen_set_env_resets(plen_ctx *ctx, const float *qpos_dev, const float *qvel_dev, const float *aux_dev, const float *man_dev,
+                        void *stream);
+int plen_get_env_resets(plen_ctx *ctx, float *qpos_dev, float *qvel_dev, float *aux_dev, float *obs_dev, float *man_dev,
+                        void *stream);
+int plen_clear_env_resets(plen_ctx *ctx, void *stream);
 
 /* Advance every env by n_ticks physics ticks with raw joint targets [N,18] (radians) and no env logic.
  * Replaces move_joints + p.stepSimulation (plen_env.py:746-753, :665-667); used by the parity tests. */

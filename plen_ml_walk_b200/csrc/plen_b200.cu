@@ -58,6 +58,10 @@ struct plen_ctx {
                      // command delay in ticks (word SC_LATENCY, plen_set_env_latency; read only while d_lat exists)
     float *d_mass;   // [n][MR_WORDS] per-robot body mass scales and torso payload (plen_set_env_mass; NULL until its first call)
     float *d_lat;    // [n][LAT_WORDS] per-robot command history ring (plen_set_env_latency; NULL until its first call)
+    float *d_rows;   // [n][PLEN_SNAP_WORDS] per-robot reset states, the snapshot's layout (plen_settle_env_resets /
+                     // plen_set_env_resets; NULL until the first of them and after plen_clear_env_resets: every reset then
+                     // restores d_snapshot)
+    float *d_rscr;   // [n][RSCR_WORDS] settle scratch kept with d_rows: start records [n][96], then manifolds [n][PLEN_MAN_WORDS]
     uint8_t *d_key;  // [n] contact-load sort key of the current tick (k_dyn -> k_rank)
     int *d_perm;     // [n_tiles * RANK_TILE] robots ordered by contact load inside each tile (k_rank -> k_solve)
     float *d_act, *d_obs, *d_rew;
@@ -67,12 +71,15 @@ struct plen_ctx {
     cudaStream_t pipe[PLEN_HOST_PIPE];      // pipe[0] == stream; ranges of plen_step_host / of a fanned-out small plen_step
     cudaEvent_t fan_fork, fan_join[PLEN_HOST_PIPE];
     cudaEvent_t last_work;                  // recorded by every entry point that queues work on a caller stream; plen_step_host waits for it
-    unsigned long long launches;            // kernels launched by plen_reset / plen_step / plen_step_host / plen_tick (plen_kernel_launches)
+    unsigned long long launches;            // kernels launched by plen_reset / plen_step / plen_step_host / plen_tick /
+                                            // plen_settle_env_resets (plen_kernel_launches)
     // optional per-kernel timing of plen_step (plen_profile_enable): 2*substeps+2 events per recorded step
     cudaEvent_t *prof_ev;
     int prof_cap, prof_steps;
     char err[512];
 };
+
+#define RSCR_WORDS (PLEN_STATE_WORDS + PLEN_MAN_WORDS)
 
 static char g_err[512] = "";
 
@@ -357,11 +364,12 @@ __global__ void k_get_latency(const float *__restrict__ scale, const float *__re
 }
 
 // After the last tick of an env step, one warp per robot: observation, done, reward, counters, auto-reset.
+// rows != NULL (plen_settle_env_resets / plen_set_env_resets): a robot that is reset restores its own row instead of the snapshot.
 __global__ void __launch_bounds__(DYN_WPC * 32)
 k_post(const __grid_constant__ DevConfig dc, const float *__restrict__ tab_g, float *__restrict__ state, int n,
        float *__restrict__ obs, float *__restrict__ reward, uint8_t *__restrict__ done, uint8_t *__restrict__ timeout,
        float *__restrict__ terminal_obs, const float *__restrict__ snapshot, unsigned long long *__restrict__ faults,
-       float *__restrict__ man) {
+       float *__restrict__ man, const float *__restrict__ rows) {
     DynSmem &sm = stage_table(tab_g);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int env = blockIdx.x * DYN_WPC + warp;
@@ -370,7 +378,7 @@ k_post(const __grid_constant__ DevConfig dc, const float *__restrict__ tab_g, fl
     LaneState L;
     load_record(state + (size_t)env * PLEN_STATE_WORDS, ws, L, lane);
     StepIO io{nullptr, obs + (size_t)env * PLEN_OBS, reward + env, done + env, timeout ? timeout + env : nullptr,
-              terminal_obs ? terminal_obs + (size_t)env * PLEN_OBS : nullptr, snapshot, faults,
+              terminal_obs ? terminal_obs + (size_t)env * PLEN_OBS : nullptr, rows ? rows + (size_t)env * PLEN_SNAP_WORDS : snapshot, faults,
               man ? man + (size_t)env * PLEN_MAN_WORDS : nullptr};
     env_post(dc, sm.tab, ws, L, lane, io);
     store_record(state + (size_t)env * PLEN_STATE_WORDS, ws, L, lane);
@@ -390,12 +398,15 @@ k_observe(const float *__restrict__ state, int n, float *__restrict__ obs) {
     if (lane < PLEN_OBS) obs[(size_t)env * PLEN_OBS + lane] = ws.obs[lane];
 }
 
-// PlenWalkEnv.reset (plen_env.py:558-614): copy the post-reset snapshot into the selected envs
+// PlenWalkEnv.reset (plen_env.py:558-614): copy the post-reset snapshot (or the robot's own row, rows != NULL) into the
+// selected envs
 __global__ void k_reset(float *__restrict__ state, int n, const uint8_t *__restrict__ mask,
-                        const float *__restrict__ snapshot, float *__restrict__ obs, float *__restrict__ man) {
+                        const float *__restrict__ snap, float *__restrict__ obs, float *__restrict__ man,
+                        const float *__restrict__ rows) {
     const int env = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (env >= n) return;
     if (mask && !mask[env]) return;
+    const float *snapshot = rows ? rows + (size_t)env * PLEN_SNAP_WORDS : snap;
     float *rec = state + (size_t)env * PLEN_STATE_WORDS;
     rec[lane] = snapshot[lane];
     rec[32 + lane] = snapshot[32 + lane];
@@ -412,10 +423,12 @@ __global__ void k_fill(float *__restrict__ state, int n, const float *__restrict
 }
 
 // aux = [lam_n[8], manifold bits, cnt, ds, hist_len, ep_t, last[6], sums[9], ep_ret]
-__global__ void k_get_state(const float *__restrict__ state, int n, float *qpos, float *qvel, float *aux) {
+// Record e starts at state + e * stride: PLEN_STATE_WORDS for the robots' states, PLEN_SNAP_WORDS for the reset rows, 0 to
+// broadcast the snapshot's record to every output row.
+__global__ void k_get_state(const float *__restrict__ state, int n, size_t stride, float *qpos, float *qvel, float *aux) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
-    const float *r = state + (size_t)e * PLEN_STATE_WORDS;
+    const float *r = state + (size_t)e * stride;
     if (qpos) {
         float *o = qpos + (size_t)e * PLEN_QPOS;
         for (int k = 0; k < 3; k++) o[k] = r[W_POS + k];
@@ -437,10 +450,10 @@ __global__ void k_get_state(const float *__restrict__ state, int n, float *qpos,
     }
 }
 
-__global__ void k_set_state(float *__restrict__ state, int n, const float *qpos, const float *qvel, const float *aux) {
+__global__ void k_set_state(float *__restrict__ state, int n, size_t stride, const float *qpos, const float *qvel, const float *aux) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
-    float *r = state + (size_t)e * PLEN_STATE_WORDS;
+    float *r = state + (size_t)e * stride;
     if (qpos) {
         const float *o = qpos + (size_t)e * PLEN_QPOS;
         for (int k = 0; k < 3; k++) r[W_POS + k] = o[k];
@@ -460,6 +473,52 @@ __global__ void k_set_state(float *__restrict__ state, int n, const float *qpos,
         for (int k = 0; k < 9; k++) r[W_SUMS + k] = o[19 + k];
         r[W_EPRET] = o[28];
     }
+}
+
+// ---- per-robot reset rows (plen_settle_env_resets / plen_set_env_resets / plen_get_env_resets)
+// width words of n rows: dst[e * dpitch + w] = src[e * spitch + w]; spitch 0 broadcasts one row.  One thread per word.
+__global__ void k_copy_rows(const float *__restrict__ src, size_t spitch, float *__restrict__ dst, size_t dpitch, int width, int n) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)n * width) return;
+    const size_t e = i / width, w = i % width;
+    dst[e * dpitch + w] = src[e * spitch + w];
+}
+
+// settle start: robot e's record at its start pose (start [n][4] = x, y, z, yaw; NULL: cfg.start_pos, yaw 0) and empty sole
+// manifolds.  One thread per robot.
+__global__ void k_start_records(const float *__restrict__ start, int n, float x0, float y0, float z0, float *__restrict__ state,
+                                float *__restrict__ man) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    if (start) {
+        const float *p = start + 4 * (size_t)e;
+        start_record(p[0], p[1], p[2], p[3], state + (size_t)e * PLEN_STATE_WORDS);
+    } else {
+        start_record(x0, y0, z0, 0.0f, state + (size_t)e * PLEN_STATE_WORDS);
+    }
+    for (int w = 0; w < PLEN_MAN_WORDS; w++) man[(size_t)e * PLEN_MAN_WORDS + w] = 0.0f;
+}
+
+// one warp per robot: the record at state + e * stride and its observation (observe, as the snapshot's is computed) into row e;
+// man != NULL also copies the robot's sole manifold.  state may be the rows themselves (the record is then rewritten as it is).
+__global__ void __launch_bounds__(DYN_WPC * 32)
+k_pack_rows(const float *state, size_t stride, const float *__restrict__ man, int n, float *rows) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    DynSmem &sm = *reinterpret_cast<DynSmem *>(smem_raw);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int env = blockIdx.x * DYN_WPC + warp;
+    if (env >= n) return;
+    WarpScratch &ws = sm.ws[warp];
+    LaneState L;
+    load_record(state + (size_t)env * stride, ws, L, lane);
+    observe(ws, L, lane);
+    float *row = rows + (size_t)env * PLEN_SNAP_WORDS;
+    row[lane] = ws.st[lane];
+    row[32 + lane] = ws.st[32 + lane];
+    row[64 + lane] = ws.st[64 + lane];
+    row[PLEN_STATE_WORDS + lane] = lane < PLEN_OBS ? ws.obs[lane] : 0.0f;     // the padding stays 0, as in the snapshot
+    if (man)
+        for (int w = lane; w < PLEN_MAN_WORDS; w += 32) row[PLEN_SNAP_MAN + w] = man[(size_t)env * PLEN_MAN_WORDS + w];
 }
 
 // ---- sinewave gait + closed-form leg IK, float64, one thread per parameter set
@@ -618,9 +677,10 @@ static void launch_dyn(plen_ctx *ctx, const float *state, int n, const float *ac
 }
 
 // n_ticks physics ticks of 1/240 s: (k_dyn, k_solve) per tick.  `actions` (agent space) only on the first tick.
+// man: the persistent sole manifolds of these robots (NULL when the context has none).
 // ev (nullable): 2*n_ticks events recorded before each kernel.
 static void launch_ticks(plen_ctx *ctx, float *state, int n, const float *actions, float *tgt, int n_ticks, cudaStream_t st,
-                         cudaEvent_t *ev = nullptr, size_t off = 0) {
+                         float *man, cudaEvent_t *ev = nullptr, size_t off = 0) {
     // off: first robot of the range inside the context's per-robot scratch (solve records, sort keys, permutation);
     // state / actions / tgt are already offset by the caller.  Ranges start on RANK_TILE boundaries.
     float *srec = ctx->d_srec + off * SR_WORDS;
@@ -629,9 +689,8 @@ static void launch_ticks(plen_ctx *ctx, float *state, int n, const float *action
     const bool boxes = ctx->dc.link_contacts != 0;
     float *srx = boxes ? ctx->d_srx + off * XR_WORDS : nullptr;
     int *xg = boxes ? ctx->d_xgroups + off / RANK_TILE : nullptr;
-    // persistent sole manifolds: the snapshot robot keeps its own behind its record
-    float *man = !ctx->d_man ? nullptr : (state == ctx->d_snapshot ? ctx->d_snapshot + PLEN_SNAP_MAN : ctx->d_man + off * PLEN_MAN_WORDS);
-    // per-robot scales and mass rows: never for the snapshot robot, which is settled under the nominal parameters
+    // per-robot scales and mass rows: never for the snapshot robot, which is settled under the nominal parameters (the
+    // robots' own reset rows, settled on the scratch state, do use them)
     const bool snap = state == ctx->d_snapshot;
     const float *scale = (snap || !ctx->d_scale) ? nullptr : ctx->d_scale + 4 * off;
     const float *mrow = (snap || !ctx->d_mass) ? nullptr : ctx->d_mass + MR_WORDS * off;
@@ -663,12 +722,14 @@ static void launch_ticks(plen_ctx *ctx, float *state, int n, const float *action
 static void launch_step_range(plen_ctx *ctx, size_t off, int cnt, const float *actions_dev, float *obs_dev, float *reward_dev,
                               uint8_t *done_dev, uint8_t *timeout_dev, float *terminal_obs_dev, cudaStream_t st, cudaEvent_t *ev, int nev) {
     float *state = ctx->d_state + off * PLEN_STATE_WORDS;
-    launch_ticks(ctx, state, cnt, actions_dev + off * PLEN_NJ, ctx->d_tgt + off * PLEN_NJ, ctx->cfg.substeps, st, ev, off);
+    launch_ticks(ctx, state, cnt, actions_dev + off * PLEN_NJ, ctx->d_tgt + off * PLEN_NJ, ctx->cfg.substeps, st,
+                 ctx->d_man ? ctx->d_man + off * PLEN_MAN_WORDS : nullptr, ev, off);
     if (ev) cudaEventRecord(ev[nev - 2], st);
     k_post<<<dyn_grid(cnt), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->dc, ctx->d_tab, state, cnt, obs_dev + off * PLEN_OBS, reward_dev + off,
                                                          done_dev + off, timeout_dev ? timeout_dev + off : nullptr,
                                                          terminal_obs_dev ? terminal_obs_dev + off * PLEN_OBS : nullptr, ctx->d_snapshot,
-                                                         ctx->d_faults, ctx->d_man ? ctx->d_man + off * PLEN_MAN_WORDS : nullptr);
+                                                         ctx->d_faults, ctx->d_man ? ctx->d_man + off * PLEN_MAN_WORDS : nullptr,
+                                                         ctx->d_rows ? ctx->d_rows + off * PLEN_SNAP_WORDS : nullptr);
     ctx->launches += 1;
     if (ev) cudaEventRecord(ev[nev - 1], st);
 }
@@ -699,7 +760,7 @@ unsigned long long plen_kernel_launches(const plen_ctx *ctx) { return ctx ? ctx-
 void plen_destroy(plen_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    cudaFree(ctx->d_tab); cudaFree(ctx->d_state); cudaFree(ctx->d_snapshot); cudaFree(ctx->d_srec); cudaFree(ctx->d_srx); cudaFree(ctx->d_xgroups); cudaFree(ctx->d_tgt); cudaFree(ctx->d_key); cudaFree(ctx->d_perm); cudaFree(ctx->d_scale); cudaFree(ctx->d_mass); cudaFree(ctx->d_lat); cudaFree(ctx->d_man); cudaFree(ctx->d_hull);
+    cudaFree(ctx->d_tab); cudaFree(ctx->d_state); cudaFree(ctx->d_snapshot); cudaFree(ctx->d_srec); cudaFree(ctx->d_srx); cudaFree(ctx->d_xgroups); cudaFree(ctx->d_tgt); cudaFree(ctx->d_key); cudaFree(ctx->d_perm); cudaFree(ctx->d_scale); cudaFree(ctx->d_mass); cudaFree(ctx->d_lat); cudaFree(ctx->d_rows); cudaFree(ctx->d_rscr); cudaFree(ctx->d_man); cudaFree(ctx->d_hull);
     cudaFree(ctx->d_act); cudaFree(ctx->d_obs); cudaFree(ctx->d_rew); cudaFree(ctx->d_done); cudaFree(ctx->d_tmo); cudaFree(ctx->d_faults);
     for (int k = 1; k < PLEN_HOST_PIPE; k++)
         if (ctx->pipe[k]) cudaStreamDestroy(ctx->pipe[k]);
@@ -733,6 +794,7 @@ static int create_impl(plen_ctx *ctx) {
     CK(ctx, cudaFuncSetAttribute(k_dyn<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_post, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_observe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
+    CK(ctx, cudaFuncSetAttribute(k_pack_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_solve<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_solve<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_solve_x, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_X_SMEM));
@@ -784,9 +846,11 @@ static int create_impl(plen_ctx *ctx) {
     // post-reset snapshot: teleport to the start pose, zero joints and targets, settle for reset_ticks (plen_env.py:561-574)
     init_record(&ctx->cfg, rec);
     CK(ctx, cudaMemcpy(ctx->d_snapshot, rec, sizeof rec, cudaMemcpyHostToDevice));
-    launch_ticks(ctx, ctx->d_snapshot, 1, nullptr, nullptr, ctx->cfg.reset_ticks, ctx->stream);
+    // (the snapshot robot keeps its persistent sole manifolds behind its record)
+    launch_ticks(ctx, ctx->d_snapshot, 1, nullptr, nullptr, ctx->cfg.reset_ticks, ctx->stream,
+                 ctx->d_man ? ctx->d_snapshot + PLEN_SNAP_MAN : nullptr);
     k_observe<<<1, 32, DYN_SMEM, ctx->stream>>>(ctx->d_snapshot, 1, ctx->d_snapshot + PLEN_STATE_WORDS);
-    k_reset<<<(n * 32 + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_state, n, nullptr, ctx->d_snapshot, nullptr, ctx->d_man);
+    k_reset<<<(n * 32 + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_state, n, nullptr, ctx->d_snapshot, nullptr, ctx->d_man, nullptr);
     CK(ctx, cudaGetLastError());
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return PLEN_OK;
@@ -825,7 +889,8 @@ plen_ctx *plen_create(const plen_config *cfg, const plen_model *model, int n_env
 int plen_reset(plen_ctx *ctx, const uint8_t *mask_dev, float *obs_dev, void *stream) {
     if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
-    k_reset<<<(ctx->n * 32 + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ctx->d_state, ctx->n, mask_dev, ctx->d_snapshot, obs_dev, ctx->d_man);
+    k_reset<<<(ctx->n * 32 + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ctx->d_state, ctx->n, mask_dev, ctx->d_snapshot, obs_dev, ctx->d_man,
+                                                                       ctx->d_rows);
     ctx->launches += 1;
     CK(ctx, cudaGetLastError());
     CK(ctx, mark_work(ctx, (cudaStream_t)stream));
@@ -914,7 +979,7 @@ int plen_step_host(plen_ctx *ctx, const float *actions_host, float *obs_host, fl
         cudaStream_t st = ctx->pipe[used % PLEN_HOST_PIPE];
         // ordering contract (plen_b200.h): this call runs on the context's private streams, so it first waits for whatever
         // the last stream-taking entry point (reset / step / set_state / set_env_scales / set_env_mass / set_env_latency /
-        // tick) queued on the caller's stream
+        // settle_env_resets / set_env_resets / clear_env_resets / tick) queued on the caller's stream
         CK(ctx, cudaStreamWaitEvent(st, ctx->last_work, 0));
         CK(ctx, cudaMemcpyAsync(ctx->d_act + off * PLEN_NJ, actions_host + off * PLEN_NJ, sizeof(float) * PLEN_NJ * cnt,
                                 cudaMemcpyHostToDevice, st));
@@ -1011,6 +1076,97 @@ int plen_set_manifold(plen_ctx *ctx, const float *man_dev, void *stream) {
     return PLEN_OK;
 }
 
+// The per-robot reset table and its settle scratch, allocated at the first settle / set call with every row the shared snapshot
+// (so that a robot nobody settled or set resets as before).  If the table cannot be completed, it is freed again.
+static int ensure_rows(plen_ctx *ctx, cudaStream_t st) {
+    if (ctx->d_rows) return PLEN_OK;
+    const size_t n = ctx->n;
+    cudaError_t e = cudaMalloc(&ctx->d_rows, sizeof(float) * PLEN_SNAP_WORDS * n);
+    if (e == cudaSuccess) e = cudaMalloc(&ctx->d_rscr, sizeof(float) * RSCR_WORDS * n);
+    if (e == cudaSuccess) {
+        k_copy_rows<<<(unsigned)((PLEN_SNAP_WORDS * n + 255) / 256), 256, 0, st>>>(ctx->d_snapshot, 0, ctx->d_rows, PLEN_SNAP_WORDS,
+                                                                                  PLEN_SNAP_WORDS, ctx->n);
+        e = cudaGetLastError();
+    }
+    if (e != cudaSuccess) {
+        cudaFree(ctx->d_rows); cudaFree(ctx->d_rscr);
+        ctx->d_rows = ctx->d_rscr = nullptr;
+        return fail(ctx, PLEN_E_CUDA, "reset table: %s", cudaGetErrorString(e));
+    }
+    return PLEN_OK;
+}
+
+int plen_settle_env_resets(plen_ctx *ctx, const float *start_dev, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    CK(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int rc = ensure_rows(ctx, st);
+    if (rc != PLEN_OK) return rc;
+    const int n = ctx->n;
+    float *rec = ctx->d_rscr, *man = ctx->d_rscr + (size_t)PLEN_STATE_WORDS * n;
+    k_start_records<<<(n + 127) / 128, 128, 0, st>>>(start_dev, n, ctx->cfg.start_pos[0], ctx->cfg.start_pos[1],
+                                                     ctx->cfg.start_pos[2], rec, man);
+    // the reference's reset under each robot's own scales and mass rows: zero targets (tgt = NULL), no command latency (no
+    // actions), the scratch manifolds rather than the running ones, the whole batch as one range
+    launch_ticks(ctx, rec, n, nullptr, nullptr, ctx->cfg.reset_ticks, st, ctx->d_man ? man : nullptr);
+    k_pack_rows<<<dyn_grid(n), DYN_WPC * 32, DYN_SMEM, st>>>(rec, PLEN_STATE_WORDS, man, n, ctx->d_rows);
+    ctx->launches += 2;
+    CK(ctx, cudaGetLastError());
+    CK(ctx, mark_work(ctx, st));
+    return PLEN_OK;
+}
+
+int plen_set_env_resets(plen_ctx *ctx, const float *qpos_dev, const float *qvel_dev, const float *aux_dev, const float *man_dev,
+                        void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    if (man_dev && !ctx->d_man) return fail(ctx, PLEN_E_STATE, "plen_set_env_resets: the context was created with sole_manifold = 0");
+    CK(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int rc = ensure_rows(ctx, st);
+    if (rc != PLEN_OK) return rc;
+    const int n = ctx->n;
+    k_set_state<<<(n + 127) / 128, 128, 0, st>>>(ctx->d_rows, n, PLEN_SNAP_WORDS, qpos_dev, qvel_dev, aux_dev);
+    if (man_dev)
+        k_copy_rows<<<(unsigned)(((size_t)PLEN_MAN_WORDS * n + 255) / 256), 256, 0, st>>>(man_dev, PLEN_MAN_WORDS, ctx->d_rows + PLEN_SNAP_MAN,
+                                                                                        PLEN_SNAP_WORDS, PLEN_MAN_WORDS, n);
+    k_pack_rows<<<dyn_grid(n), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->d_rows, PLEN_SNAP_WORDS, nullptr, n, ctx->d_rows);   // new observations
+    CK(ctx, cudaGetLastError());
+    CK(ctx, mark_work(ctx, st));
+    return PLEN_OK;
+}
+
+int plen_get_env_resets(plen_ctx *ctx, float *qpos_dev, float *qvel_dev, float *aux_dev, float *obs_dev, float *man_dev, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    if (man_dev && !ctx->d_man) return fail(ctx, PLEN_E_STATE, "plen_get_env_resets: the context was created with sole_manifold = 0");
+    CK(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int n = ctx->n;
+    const float *src = ctx->d_rows ? ctx->d_rows : ctx->d_snapshot;
+    const size_t pitch = ctx->d_rows ? PLEN_SNAP_WORDS : 0;       // no table: the shared snapshot for every robot
+    if (qpos_dev || qvel_dev || aux_dev)
+        k_get_state<<<(n + 127) / 128, 128, 0, st>>>(src, n, pitch, qpos_dev, qvel_dev, aux_dev);
+    if (obs_dev)
+        k_copy_rows<<<(unsigned)(((size_t)PLEN_OBS * n + 255) / 256), 256, 0, st>>>(src + PLEN_STATE_WORDS, pitch, obs_dev, PLEN_OBS,
+                                                                                  PLEN_OBS, n);
+    if (man_dev)
+        k_copy_rows<<<(unsigned)(((size_t)PLEN_MAN_WORDS * n + 255) / 256), 256, 0, st>>>(src + PLEN_SNAP_MAN, pitch, man_dev,
+                                                                                        PLEN_MAN_WORDS, PLEN_MAN_WORDS, n);
+    CK(ctx, cudaGetLastError());
+    return ctx->d_rows ? 1 : 0;
+}
+
+int plen_clear_env_resets(plen_ctx *ctx, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    if (!ctx->d_rows) return PLEN_OK;
+    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, cudaStreamSynchronize((cudaStream_t)stream));     // steps queued before this call still read the rows
+    const cudaError_t e0 = cudaFree(ctx->d_rows), e1 = cudaFree(ctx->d_rscr);
+    ctx->d_rows = ctx->d_rscr = nullptr;
+    CK(ctx, e0 != cudaSuccess ? e0 : e1);
+    CK(ctx, mark_work(ctx, (cudaStream_t)stream));
+    return PLEN_OK;
+}
+
 int plen_fault_count(plen_ctx *ctx, unsigned long long *count_host) {
     if (!ctx || !count_host) return fail(ctx, PLEN_E_ARG, "plen_fault_count: bad arguments");
     CK(ctx, cudaSetDevice(ctx->device));
@@ -1022,7 +1178,7 @@ int plen_fault_count(plen_ctx *ctx, unsigned long long *count_host) {
 int plen_get_state(plen_ctx *ctx, float *qpos_dev, float *qvel_dev, float *aux_dev, void *stream) {
     if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
-    k_get_state<<<(ctx->n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ctx->d_state, ctx->n, qpos_dev, qvel_dev, aux_dev);
+    k_get_state<<<(ctx->n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ctx->d_state, ctx->n, PLEN_STATE_WORDS, qpos_dev, qvel_dev, aux_dev);
     CK(ctx, cudaGetLastError());
     return PLEN_OK;
 }
@@ -1030,7 +1186,7 @@ int plen_get_state(plen_ctx *ctx, float *qpos_dev, float *qvel_dev, float *aux_d
 int plen_set_state(plen_ctx *ctx, const float *qpos_dev, const float *qvel_dev, const float *aux_dev, void *stream) {
     if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
-    k_set_state<<<(ctx->n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ctx->d_state, ctx->n, qpos_dev, qvel_dev, aux_dev);
+    k_set_state<<<(ctx->n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ctx->d_state, ctx->n, PLEN_STATE_WORDS, qpos_dev, qvel_dev, aux_dev);
     CK(ctx, cudaGetLastError());
     CK(ctx, mark_work(ctx, (cudaStream_t)stream));
     return PLEN_OK;
@@ -1043,7 +1199,7 @@ int plen_tick(plen_ctx *ctx, const float *targets_dev, int n_ticks, void *stream
     if (targets_dev)
         CK(ctx, cudaMemcpyAsync(ctx->d_tgt, targets_dev, sizeof(float) * PLEN_NJ * (size_t)ctx->n, cudaMemcpyDeviceToDevice,
                                 (cudaStream_t)stream));
-    launch_ticks(ctx, ctx->d_state, ctx->n, nullptr, targets_dev ? ctx->d_tgt : nullptr, n_ticks, (cudaStream_t)stream);
+    launch_ticks(ctx, ctx->d_state, ctx->n, nullptr, targets_dev ? ctx->d_tgt : nullptr, n_ticks, (cudaStream_t)stream, ctx->d_man);
     CK(ctx, cudaGetLastError());
     CK(ctx, mark_work(ctx, (cudaStream_t)stream));
     return PLEN_OK;

@@ -77,9 +77,22 @@ PLEN_DEV void observe(WarpScratch &ws, const LaneState &L, int lane) {
     warp_sync();
 }
 
-// post-reset snapshot: record (96) | observation (26, padded to 32) | sole manifolds (PLEN_MAN_WORDS)
+// post-reset snapshot: record (96) | observation (26, padded to 32) | sole manifolds (PLEN_MAN_WORDS).  The per-robot reset rows
+// of plen_settle_env_resets / plen_set_env_resets have the same layout, one row per robot.
 #define PLEN_SNAP_MAN (PLEN_STATE_WORDS + 32)
 #define PLEN_SNAP_WORDS (PLEN_SNAP_MAN + PLEN_MAN_WORDS)
+
+// Record of a robot teleported to base position (x, y, z) with heading yaw about world z, quaternion (0, 0, sin(yaw/2),
+// cos(yaw/2)): zero joints, velocities, contact cache and bookkeeping (plen_env.py:561-565), before the settle ticks.
+// init_record (plen_host_tables.h) is the case cfg.start_pos, yaw 0.  The half-angle sine and cosine are taken in double and
+// rounded once, so that a host building the same quaternion in float64 gets the same float32 words.
+PLEN_DEV void start_record(float x, float y, float z, float yaw, float *rec /* [96] */) {
+    for (int w = 0; w < PLEN_STATE_WORDS; w++) rec[w] = 0.0f;
+    rec[W_POS] = x; rec[W_POS + 1] = y; rec[W_POS + 2] = z;
+    const double h = 0.5 * (double)yaw;
+    rec[W_QUAT + 2] = (float)sin(h);
+    rec[W_QUAT + 3] = (float)cos(h);
+}
 
 struct StepIO {
     const float *action;      // [18] this env
@@ -87,7 +100,7 @@ struct StepIO {
     float *reward;            // scalar
     uint8_t *done, *timeout;  // scalars (timeout nullable)
     float *terminal_obs;      // [26] nullable
-    const float *snapshot;    // [96 + 26] post-reset record and its observation
+    const float *snapshot;    // [96 + 26] post-reset record and its observation: the shared snapshot or the robot's own reset row
     unsigned long long *faults;   // device counter of numeric faults (nullable)
     float *man;               // this robot's persistent sole manifold (sole_manifold = 1), nullable: reset with the record
 };
@@ -226,7 +239,8 @@ PLEN_DEV void env_post(const DevConfig &cfg, const float *tab, WarpScratch &ws, 
     warp_sync();
     if ((done && cfg.auto_reset) || fault) {
         // the reference caller resets after a terminal step (plen_td3.py:122-129); the reset is deterministic
-        // (fixed pose + 8 ticks, plen_env.py:561-570) so the post-reset record is a constant snapshot
+        // (fixed pose + 8 ticks, plen_env.py:561-570) so the post-reset record is precomputed: the shared snapshot, or the
+        // robot's own row settled under its parameters (plen_settle_env_resets)
         if (io.terminal_obs && lane < 26) io.terminal_obs[lane] = fault ? io.snapshot[96 + lane] : ws.obs[lane];
         load_record(io.snapshot, ws, L, lane);
         if (lane < 26) io.obs[lane] = io.snapshot[96 + lane];

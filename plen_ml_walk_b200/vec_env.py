@@ -215,8 +215,9 @@ class PlenVecEnv:
         """Per-env domain randomisation (SURVEY.md 8f-3): scale factors [N] of the foot friction coefficients, the servo force
         limit and the servo position gain; None leaves a quantity unchanged, 1.0 is the reference's constant.
 
-        Approximation: a reset (explicit or in-kernel auto-reset) restores the ONE post-reset snapshot that was settled for 8
-        ticks under unit scales at creation, whatever the robot's own scales are; its first steps then run under its scales."""
+        Resets: by default a reset (explicit or in-kernel auto-reset) restores the ONE post-reset snapshot that was settled for
+        8 ticks under unit scales at creation, whatever the robot's own scales are; its first steps then run under its scales.
+        Call settle_resets() after the setters to settle every robot's reset state under its own scales instead."""
         arr = [None if x is None else self._dev_f32(x, (self.num_envs,)) for x in (friction, motor_force, motor_gain)]
         for k, x in zip(("friction", "motor_force", "motor_gain"), arr):
             if x is not None:
@@ -241,8 +242,9 @@ class PlenVecEnv:
         Before the first call every robot has scale 1 and payload 0, and such a robot steps bit-identically to a context that
         never called this.  Takes effect from the next tick.
 
-        Approximation, as for set_env_scales: a reset (explicit or in-kernel auto-reset) restores the ONE post-reset snapshot
-        settled under the nominal model at creation; the robot's own masses apply from its first tick after that."""
+        Resets, as for set_env_scales: by default a reset (explicit or in-kernel auto-reset) restores the ONE post-reset
+        snapshot settled under the nominal model at creation, and the robot's own masses apply from its first tick after that.
+        Call settle_resets() after the setters to settle every robot's reset state under its own masses instead."""
         n = self.num_envs
         s = p = None
         if mass_scale is not None:
@@ -325,16 +327,81 @@ class PlenVecEnv:
         """-> int32 [N]: each robot's command delay in physics ticks (0 where set_env_latency was never called)."""
         return self._get_env_latency()[0]
 
+    def settle_resets(self, start_pose=None):
+        """Per-env reset states (no reference counterpart): run the reference's reset procedure (plen_env.py:558-574) for every
+        robot under its current friction / force / gain scales and masses, and make the result the state that robot's resets
+        (reset(), the in-kernel auto-reset, the numeric guard) restore from now on.
+
+        start_pose: None (the reference's start position, heading 0), [4] for every robot or [N,4]: (x, y, z, yaw) -- base
+                    position in the world (m) and heading about world z (rad).  Each robot is teleported there with zero
+                    joints, velocities and targets, empty contact caches, and settled for reset_ticks (8) ticks with hold
+                    target 0.  Raises ValueError on a wrong shape or a non-finite value.
+        Intended workflow: set the domain-randomisation parameters (set_env_scales, set_env_mass), call settle_resets(), then
+        reset() if the robots should start from their new reset states now -- the running states are not touched, a new
+        reset state applies from each robot's next reset.  Command latency does not act during the settle (raw physics, like
+        tick()).  A nominal robot settled from the default pose gets exactly the shared snapshot."""
+        n = self.num_envs
+        p = None
+        if start_pose is not None:
+            p = torch.as_tensor(start_pose, dtype=torch.float32, device=self.device)
+            if tuple(p.shape) == (4,):
+                p = p[None, :].expand(n, 4)
+            p = self._dev_f32(p, (n, 4))
+            if not bool(torch.isfinite(p).all()):
+                raise ValueError("start_pose must be finite")
+        with torch.cuda.device(self.device):
+            self._check(self.lib.plen_settle_env_resets(self._ctx, self._p(p), self._stream()))
+
+    def set_env_resets(self, qpos=None, qvel=None, aux=None, man=None):
+        """User-supplied reset states (recorded states, curricula) in the layouts of set_state / set_manifold; None leaves that
+        part of every robot's reset state as it is (the shared snapshot before the first settle_resets / set_env_resets).  The
+        observation of each reset state is computed from it.  man needs config_overrides={"sole_manifold": 1}."""
+        n = self.num_envs
+        qpos = None if qpos is None else self._dev_f32(qpos, (n, 25))
+        qvel = None if qvel is None else self._dev_f32(qvel, (n, 24))
+        aux = None if aux is None else self._dev_f32(aux, (n, _abi.AUX_WORDS))
+        man = None if man is None else self._dev_f32(man, (n, _abi.MAN_WORDS))
+        with torch.cuda.device(self.device):
+            self._check(self.lib.plen_set_env_resets(self._ctx, self._p(qpos), self._p(qvel), self._p(aux), self._p(man),
+                                                     self._stream()))
+
+    def _get_env_resets(self):
+        n, dev = self.num_envs, self.device
+        qpos = torch.empty((n, 25), dtype=torch.float32, device=dev)
+        qvel = torch.empty((n, 24), dtype=torch.float32, device=dev)
+        aux = torch.empty((n, _abi.AUX_WORDS), dtype=torch.float32, device=dev)
+        obs = torch.empty((n, OBS_DIM), dtype=torch.float32, device=dev)
+        man = torch.empty((n, _abi.MAN_WORDS), dtype=torch.float32, device=dev) if int(self.cfg.sole_manifold) else None
+        with torch.cuda.device(self.device):
+            rc = self.lib.plen_get_env_resets(self._ctx, self._p(qpos), self._p(qvel), self._p(aux), self._p(obs), self._p(man),
+                                              self._stream())
+        if rc < 0:
+            self._check(rc)
+        return (qpos, qvel, aux, obs, man), rc == 1
+
+    def get_env_resets(self):
+        """-> (qpos [N,25], qvel [N,24], aux [N,29], obs [N,26], man [N,52] or None without sole_manifold): the state each
+        robot's next reset restores (the shared snapshot where no settle_resets / set_env_resets has been called)."""
+        return self._get_env_resets()[0]
+
+    def clear_env_resets(self):
+        """Drop the per-env reset states: every reset restores the shared snapshot again, exactly as on a fresh env."""
+        with torch.cuda.device(self.device):
+            self._check(self.lib.plen_clear_env_resets(self._ctx, self._stream()))
+
     def save_state(self, path):
-        """Snapshot of every env (pose, velocities, contact cache, env bookkeeping, per-env scales, masses, command delays and
-        command history) to one .pt file (SURVEY.md 8f-4)."""
+        """Snapshot of every env (pose, velocities, contact cache, env bookkeeping, per-env scales, masses, command delays,
+        command history and reset states) to one .pt file (SURVEY.md 8f-4)."""
         qpos, qvel, aux = self.get_state()
         ms, mp, mass_set = self._get_env_mass()
         lt, lh, lat_set = self._get_env_latency()
+        rows, rows_set = self._get_env_resets()
         torch.save({"num_envs": self.num_envs, "joint_act": self.joint_act, "qpos": qpos.cpu(), "qvel": qvel.cpu(), "aux": aux.cpu(),
                     "scales": {k: v.cpu() for k, v in self._scales.items()},
                     "mass": {"scale": ms.cpu(), "payload": mp.cpu()} if mass_set else None,
                     "latency": {"ticks": lt.cpu(), "history": lh.cpu()} if lat_set else None,
+                    "resets": dict(zip(("qpos", "qvel", "aux", "man"), (None if t is None else t.cpu() for t in rows[:3] + rows[4:])))
+                    if rows_set else None,
                     "manifold": self.get_manifold().cpu() if int(self.cfg.sole_manifold) else None}, path)
 
     def load_state(self, path):
@@ -359,6 +426,11 @@ class PlenVecEnv:
             self.set_env_latency(lat["ticks"], lat["history"])
         elif self._get_env_latency()[2]:
             self.set_env_latency(0)
+        rows = d.get("resets")
+        if rows is not None:        # reset states likewise; a snapshot without them leaves the context on the shared snapshot
+            self.set_env_resets(rows["qpos"], rows["qvel"], rows["aux"], rows["man"])
+        else:
+            self.clear_env_resets()
 
     def tick(self, targets, n_ticks=1):
         """Raw physics: n_ticks of 1/240 s with joint targets in radians, no env logic (move_joints + stepSimulation)."""

@@ -10,11 +10,18 @@ noise to give a distribution.  Reports episode length / return of the first epis
 
     python scripts/walk_eval_batched.py [--envs 4096] [--sigma 0.05] [--precision fp32|fp16]
                                         [--mass-scale S] [--payload KG [--payload-offset X Y Z]] [--latency-ticks D | LO:HI]
+                                        [--settle-resets] [--start-pose X Y Z YAW]
 
 --mass-scale / --payload sweep the policy's robustness to the robot's mass (PlenVecEnv.set_env_mass): every body x S, and a
 point mass of KG kg on the torso, by default at the torso body's centre of mass.  --latency-ticks sweeps its robustness to servo
 command latency (PlenVecEnv.set_env_latency): every robot's servos act D physics ticks (4.17 ms each at 240 Hz) late, or a
 delay drawn uniformly from LO..HI per robot (seeded).
+
+--settle-resets settles every robot's reset state under its own masses and scales (PlenVecEnv.settle_resets, after the mass and
+latency setters, before reset()); without it a robot starts from the one snapshot settled under the nominal model.
+--start-pose settles every robot from base position (X, Y, Z) with heading YAW about world z instead of the reference's start
+(implies --settle-resets).  The distance walked is reported as the distance of the base from its settled start position in the
+ground plane, alongside the final x.
 """
 import argparse
 import json
@@ -47,6 +54,10 @@ def main():
                     help="where the payload sits in the torso body frame, m (default: the torso's centre of mass)")
     ap.add_argument("--latency-ticks", default=None, metavar="D|LO:HI",
                     help="servo command latency in physics ticks (0 .. 2 * substeps), or LO:HI for a uniform draw per robot")
+    ap.add_argument("--settle-resets", action="store_true",
+                    help="settle each robot's reset state under its own masses and scales before the rollouts")
+    ap.add_argument("--start-pose", type=float, nargs=4, default=None, metavar=("X", "Y", "Z", "YAW"),
+                    help="start every robot from this base position (m) and heading (rad); implies --settle-resets")
     a = ap.parse_args()
     dev = torch.device("cuda:0")
     g = np.load(GOLD)
@@ -71,10 +82,14 @@ def main():
         gen = torch.Generator(device=dev); gen.manual_seed(0)
         env.set_env_latency(torch.randint(lo, hi + 1, (n,), device=dev, generator=gen))
         latency = {"ticks_lo": lo, "ticks_hi": hi, "ms_per_tick": 1000.0 * float(env.cfg.dt)}
+    settle = a.settle_resets or a.start_pose is not None
+    if settle:
+        env.settle_resets(start_pose=a.start_pose)
     state = env.reset().clone()
+    xy0 = env.get_state()[0][:, 0:2].clone()
     alive = torch.ones(n, dtype=torch.bool, device=dev)
     ep_len = torch.zeros(n, device=dev); ep_ret = torch.zeros(n, device=dev)
-    x_end = torch.zeros(n, device=dev)
+    x_end = torch.zeros(n, device=dev); d_end = torch.zeros(n, device=dev)
     for t in range(a.steps):
         act = actor_forward(actor, state, noise_std=a.sigma, seed=t + 1, precision=a.precision)
         clean = actor_forward(actor, state[:1], precision=a.precision)
@@ -84,17 +99,21 @@ def main():
         ep_ret += torch.where(alive, r, torch.zeros_like(r))
         qpos = env.get_state()[0]
         x_end = torch.where(alive, qpos[:, 0], x_end)
+        d_end = torch.where(alive, (qpos[:, 0:2] - xy0).norm(dim=1), d_end)
         alive &= ~done
         state = obs.clone()
-    L, R, X = ep_len.cpu().numpy(), ep_ret.cpu().numpy(), x_end.cpu().numpy()
+    L, R, X, D = ep_len.cpu().numpy(), ep_ret.cpu().numpy(), x_end.cpu().numpy(), d_end.cpu().numpy()
     print(json.dumps({
         "policy": "plen_walk_gazebo_3229999 (reference checkpoint)", "envs": n, "steps": a.steps, "sigma": a.sigma,
         "precision": a.precision, "sole_manifold": a.sole_manifold, "config_overrides": ovr, "mass": mass, "latency": latency,
-        "deterministic": {"episode_length": float(L[0]), "return": float(R[0]), "x_final_m": float(X[0])},
+        "settled_resets": settle, "start_pose": a.start_pose,
+        "deterministic": {"episode_length": float(L[0]), "return": float(R[0]), "x_final_m": float(X[0]),
+                          "distance_from_start_m": float(D[0])},
         "noisy": {"episode_length_mean": float(L[1:].mean()), "episode_length_median": float(np.median(L[1:])),
                   "survived_all_steps_frac": float((L[1:] >= a.steps).mean()), "return_mean": float(R[1:].mean()),
                   "return_quantiles_5_25_50_75_95": [float(q) for q in np.quantile(R[1:], [0.05, 0.25, 0.5, 0.75, 0.95])],
-                  "x_final_mean_m": float(X[1:].mean()), "x_final_std_m": float(X[1:].std())}}))
+                  "x_final_mean_m": float(X[1:].mean()), "x_final_std_m": float(X[1:].std()),
+                  "distance_from_start_mean_m": float(D[1:].mean()), "distance_from_start_std_m": float(D[1:].std())}}))
 
 
 if __name__ == "__main__":
