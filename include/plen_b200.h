@@ -167,8 +167,8 @@ int plen_step(plen_ctx *ctx, const float *actions_dev, float *obs_dev, float *re
  * and a stream synchronise.  This is the end-to-end path a PyBullet user would see.
  * Ordering contract: the call runs on the context's PRIVATE streams (the batch is pipelined in ranges).  It first waits
  * (cudaStreamWaitEvent) for the work the last plen_reset / plen_step / plen_set_state / plen_set_manifold / plen_set_env_scales /
- * plen_set_env_mass / plen_set_env_latency / plen_settle_env_resets / plen_set_env_resets / plen_clear_env_resets / plen_tick call
- * queued on its caller stream, so `plen_reset(...); plen_step_host(...)`
+ * plen_set_env_mass / plen_set_env_latency / plen_settle_env_resets / plen_set_env_resets / plen_clear_env_resets /
+ * plen_set_env_obs_noise / plen_set_env_obs_noise_state / plen_clear_env_obs_noise / plen_tick call queued on its caller stream, so `plen_reset(...); plen_step_host(...)`
  * needs no synchronisation in between; it
  * returns after its own streams have drained, so whatever the caller queues next is ordered after it.  (Work the caller
  * queued on a stream WITHOUT going through this library -- e.g. a torch kernel still writing the state through
@@ -273,6 +273,56 @@ int plen_set_env_resets(plen_ctx *ctx, const float *qpos_dev, const float *qvel_
 int plen_get_env_resets(plen_ctx *ctx, float *qpos_dev, float *qvel_dev, float *aux_dev, float *obs_dev, float *man_dev,
                         void *stream);
 int plen_clear_env_resets(plen_ctx *ctx, void *stream);
+
+/* Per-env observation noise (SURVEY.md 8f-3, sensing side; the reference has none): the observations the library hands to the
+ * agent -- obs of plen_step / plen_step_host / plen_reset and terminal_obs -- carry sensor noise.  Reward, done, timeout, the
+ * gait counters, the state record and the physics keep using the true state.  For robot e, continuous words w = 0..23
+ * (q1..q18, z, vx, roll, pitch, yaw, y) and the contact flags w = 24, 25:
+ *   noisy_w = clean_w + fmaf(sigma_w, n, b_w)    n ~ N(0,1) fresh for every observation; where sigma_w == 0 and b_w == 0 the
+ *                                               word is passed through bit for bit (-0.0 and NaN included).  No clipping, no
+ *                                               angle wrapping: roll / pitch / yaw may leave [-pi, pi], z may go negative.
+ *   b_w = beta_w * n'                           per-episode bias, drawn at every reset of the robot (plen_reset for the masked
+ *                                               robots, the auto-reset, the numeric guard's forced reset) and constant for
+ *                                               the episode: its reset observation, every observation and its terminal_obs
+ *                                               carry it.
+ *   flag -> 1 - flag                            independently per observation with probability p.
+ * Draws are counter-based and stateless given a per-robot draw counter in device memory, which k_post increments once per step
+ * and k_reset once per robot it resets -- so a CUDA graph that captures plen_step draws new noise on every replay.  With
+ * gid = first_env_id + e, mix64 the splitmix64 finaliser (x += 0x9E3779B97F4A7C15; x = (x ^ x >> 30) * 0xBF58476D1CE4E5B9;
+ * x = (x ^ x >> 27) * 0x94D049BB133111EB; x ^ x >> 31) and hash32(k) = mix64(k) >> 32, all in uint64:
+ *   k  = mix64(seed ^ mix64(gid)) + (counter << 8) + (s << 5) + w
+ *   n  = sqrtf(-2 logf(u1)) * cospif(2 u2),  u1 = ((float)hash32(k) + 1) * 2.3283064e-10f,
+ *        u2 = (float)hash32(k ^ 0xA5A5A5A5DEADBEEF) * 2.3283064e-10f        (float32 arithmetic; plen_actor_forward's generator)
+ *   flip where (uint64)hash32(k) < (uint64)((double)p * 2^32)
+ * Streams s: 0 the step's observation noise (also its terminal_obs), 1 the step's flips, 2 the new episode's bias, 3 the
+ * noise of a reset observation, 4 its flips.  The draws depend neither on a robot's position in the batch nor on how
+ * plen_step / plen_step_host cut it into ranges: a sharded caller passes its shard's first global robot id as first_env_id
+ * and gets the noise of one big context.
+ *
+ * plen_set_env_obs_noise: sigma_dev [N,24] (>= 0), bias_std_dev [N,24] beta (>= 0), flip_dev [N] p (in [0,1]) device floats;
+ * NULL leaves a part as it is.  seed and first_env_id (>= 0, else PLEN_E_ARG) are set by every call; a captured graph keeps
+ * the values of its capture.  The first call allocates the noise rows (384 bytes per robot) and two clean-observation buffers
+ * (2 x 104 bytes per robot), zeroes every sigma, beta, p, bias and counter, and switches k_post to its noise instance;
+ * episodes already running keep b = 0, so the bias applies from each robot's next reset.  Graphs captured before the first
+ * call keep the stock kernel.  Precondition (not checked here, PlenVecEnv.set_obs_noise checks it): finite values in those
+ * ranges; a NaN sigma makes NaN observations, a p outside [0,1] acts as 0 or 1.
+ * plen_set_env_obs_noise_state: the running biases bias_dev [N,24] and draw counters counter_dev [N] (uint32), NULL leaves a
+ * part as it is; for snapshots that must continue bit for bit.  PLEN_E_STATE without a table.
+ * plen_get_env_obs_noise: the parameters, biases and counters into device buffers of the same layouts, seed and first_env_id
+ * into host variables; any pointer may be NULL.  Returns 1 when the context has a table, 0 when not (the buffers then receive
+ * zeros), < 0 on error.
+ * plen_clear_env_obs_noise: synchronises `stream` and frees the table; the context is then exactly the stock path again.
+ * plen_get_clean_obs: the noise-free observations [N,26] of the last step or reset (what a context without noise would have
+ * written to obs) and the noise-free terminal observations [N,26] (written where a step reported done, whether or not that
+ * step was given a terminal_obs buffer); either pointer may be NULL.  Both are zero until the first step or reset after the
+ * first plen_set_env_obs_noise.  For asymmetric actor-critic training.  PLEN_E_STATE without a table. */
+int plen_set_env_obs_noise(plen_ctx *ctx, const float *sigma_dev, const float *bias_std_dev, const float *flip_dev,
+                           unsigned long long seed, long long first_env_id, void *stream);
+int plen_set_env_obs_noise_state(plen_ctx *ctx, const float *bias_dev, const uint32_t *counter_dev, void *stream);
+int plen_get_env_obs_noise(plen_ctx *ctx, float *sigma_dev, float *bias_std_dev, float *flip_dev, float *bias_dev,
+                           uint32_t *counter_dev, unsigned long long *seed, long long *first_env_id, void *stream);
+int plen_clear_env_obs_noise(plen_ctx *ctx, void *stream);
+int plen_get_clean_obs(plen_ctx *ctx, float *obs_dev, float *terminal_obs_dev, void *stream);
 
 /* Advance every env by n_ticks physics ticks with raw joint targets [N,18] (radians) and no env logic.
  * Replaces move_joints + p.stepSimulation (plen_env.py:746-753, :665-667); used by the parity tests. */

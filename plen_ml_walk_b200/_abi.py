@@ -94,7 +94,9 @@ def model_to_c(model: PlenModel) -> PlenModelC:
 
 EXPORTS = (
     "plen_version", "plen_default_config", "plen_create", "plen_destroy", "plen_last_error", "plen_num_envs", "plen_kernel_launches",
-    "plen_reset", "plen_step", "plen_step_host", "plen_fault_count", "plen_get_state", "plen_set_state", "plen_set_env_scales", "plen_set_env_mass", "plen_get_env_mass", "plen_set_env_latency", "plen_get_env_latency", "plen_settle_env_resets", "plen_set_env_resets", "plen_get_env_resets", "plen_clear_env_resets", "plen_get_manifold", "plen_set_manifold", "plen_tick",
+    "plen_reset", "plen_step", "plen_step_host", "plen_fault_count", "plen_get_state", "plen_set_state", "plen_set_env_scales", "plen_set_env_mass", "plen_get_env_mass", "plen_set_env_latency", "plen_get_env_latency", "plen_settle_env_resets", "plen_set_env_resets", "plen_get_env_resets", "plen_clear_env_resets",
+    "plen_set_env_obs_noise", "plen_set_env_obs_noise_state", "plen_get_env_obs_noise", "plen_clear_env_obs_noise", "plen_get_clean_obs",
+    "plen_get_manifold", "plen_set_manifold", "plen_tick",
     "plen_debug_dynamics", "plen_debug_records", "plen_gait_ik", "plen_profile_enable", "plen_profile_read", "plen_measure_fp32_peak",
     "plen_replay_create", "plen_replay_destroy", "plen_replay_size", "plen_replay_ptr", "plen_replay_storage",
     "plen_replay_add", "plen_replay_sample", "plen_actor_forward", "plen_actor_forward_tc", "plen_actor_tc_timed_out", "plen_td3_last_error", "plen_td3_set_precision", "plen_td3_tc_timed_out",
@@ -156,6 +158,11 @@ def load_library(path: str = LIB_PATH):
     L.plen_set_env_resets.argtypes = [vp] * 6
     L.plen_get_env_resets.argtypes = [vp] * 7
     L.plen_clear_env_resets.argtypes = [vp] * 2
+    L.plen_set_env_obs_noise.argtypes = [vp] * 4 + [C.c_ulonglong, C.c_longlong, vp]
+    L.plen_set_env_obs_noise_state.argtypes = [vp] * 4
+    L.plen_get_env_obs_noise.argtypes = [vp] * 6 + [C.POINTER(C.c_ulonglong), C.POINTER(C.c_longlong), vp]
+    L.plen_clear_env_obs_noise.argtypes = [vp] * 2
+    L.plen_get_clean_obs.argtypes = [vp] * 4
     L.plen_tick.argtypes = [vp, vp, ip, vp]
     L.plen_get_manifold.argtypes = [vp, vp, vp]
     L.plen_set_manifold.argtypes = [vp, vp, vp]

@@ -62,6 +62,11 @@ struct plen_ctx {
                      // plen_set_env_resets; NULL until the first of them and after plen_clear_env_resets: every reset then
                      // restores d_snapshot)
     float *d_rscr;   // [n][RSCR_WORDS] settle scratch kept with d_rows: start records [n][96], then manifolds [n][PLEN_MAN_WORDS]
+    float *d_noise;  // [n][ON_WORDS] per-robot observation noise rows (plen_set_env_obs_noise; NULL until its first call and after
+                     // plen_clear_env_obs_noise: k_post's stock instance runs then)
+    float *d_cobs, *d_ctobs;   // [n][26] each: noise-free obs / terminal obs of the last step or reset (kept with d_noise)
+    unsigned long long noise_seed;
+    long long noise_first;     // global id of robot 0 (a shard's first robot): draws are keyed by first + robot
     uint8_t *d_key;  // [n] contact-load sort key of the current tick (k_dyn -> k_rank)
     int *d_perm;     // [n_tiles * RANK_TILE] robots ordered by contact load inside each tile (k_rank -> k_solve)
     float *d_act, *d_obs, *d_rew;
@@ -363,13 +368,48 @@ __global__ void k_get_latency(const float *__restrict__ scale, const float *__re
     }
 }
 
+// per-robot observation noise rows, one thread per word: sigma [n][24], bias std [n][24], flip [n]; NULL leaves a part as it is,
+// `init` first zeroes the whole row (no noise, bias 0, counter 0).  bias [n][24] and counter [n] (uint32) are the running state.
+__global__ void k_set_obs_noise(float *__restrict__ row, int n, const float *sigma, const float *beta, const float *flip,
+                                const float *bias, const unsigned *counter, int init) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)n * ON_WORDS) return;
+    const size_t e = i / ON_WORDS;
+    const int w = (int)(i % ON_WORDS);
+    if (init) row[i] = 0.0f;
+    if (sigma && w >= ON_SIGMA && w < ON_SIGMA + 24) row[i] = sigma[e * 24 + (w - ON_SIGMA)];
+    if (beta && w >= ON_BETA && w < ON_BETA + 24) row[i] = beta[e * 24 + (w - ON_BETA)];
+    if (bias && w >= ON_BIAS && w < ON_BIAS + 24) row[i] = bias[e * 24 + (w - ON_BIAS)];
+    if (flip && w == ON_FLIP) row[i] = flip[e];
+    if (counter && w == ON_CTR) row[i] = bits_f(counter[e]);
+}
+
+// ... and back; zeros when the context has no rows
+__global__ void k_get_obs_noise(const float *__restrict__ row, int n, float *sigma, float *beta, float *flip, float *bias,
+                                unsigned *counter) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)n * ON_WORDS) return;
+    const size_t e = i / ON_WORDS;
+    const int w = (int)(i % ON_WORDS);
+    const float v = row ? row[i] : 0.0f;
+    if (sigma && w >= ON_SIGMA && w < ON_SIGMA + 24) sigma[e * 24 + (w - ON_SIGMA)] = v;
+    if (beta && w >= ON_BETA && w < ON_BETA + 24) beta[e * 24 + (w - ON_BETA)] = v;
+    if (bias && w >= ON_BIAS && w < ON_BIAS + 24) bias[e * 24 + (w - ON_BIAS)] = v;
+    if (flip && w == ON_FLIP) flip[e] = v;
+    if (counter && w == ON_CTR) counter[e] = f_bits(v);
+}
+
 // After the last tick of an env step, one warp per robot: observation, done, reward, counters, auto-reset.
 // rows != NULL (plen_settle_env_resets / plen_set_env_resets): a robot that is reset restores its own row instead of the snapshot.
+// NOISE (launched only while the context has noise rows): observation noise on obs / terminal_obs, the clean words into
+// clean_obs / clean_tobs, draws keyed by (seed, gid0 + robot); the false instance is the stock path and ignores those arguments.
+template <bool NOISE>
 __global__ void __launch_bounds__(DYN_WPC * 32)
 k_post(const __grid_constant__ DevConfig dc, const float *__restrict__ tab_g, float *__restrict__ state, int n,
        float *__restrict__ obs, float *__restrict__ reward, uint8_t *__restrict__ done, uint8_t *__restrict__ timeout,
        float *__restrict__ terminal_obs, const float *__restrict__ snapshot, unsigned long long *__restrict__ faults,
-       float *__restrict__ man, const float *__restrict__ rows) {
+       float *__restrict__ man, const float *__restrict__ rows, float *__restrict__ noise, float *__restrict__ clean_obs,
+       float *__restrict__ clean_tobs, unsigned long long seed, long long gid0) {
     DynSmem &sm = stage_table(tab_g);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int env = blockIdx.x * DYN_WPC + warp;
@@ -380,7 +420,13 @@ k_post(const __grid_constant__ DevConfig dc, const float *__restrict__ tab_g, fl
     StepIO io{nullptr, obs + (size_t)env * PLEN_OBS, reward + env, done + env, timeout ? timeout + env : nullptr,
               terminal_obs ? terminal_obs + (size_t)env * PLEN_OBS : nullptr, rows ? rows + (size_t)env * PLEN_SNAP_WORDS : snapshot, faults,
               man ? man + (size_t)env * PLEN_MAN_WORDS : nullptr};
-    env_post(dc, sm.tab, ws, L, lane, io);
+    if constexpr (NOISE) {
+        io.noise = noise + (size_t)env * ON_WORDS;
+        io.clean_obs = clean_obs + (size_t)env * PLEN_OBS;
+        io.clean_tobs = clean_tobs + (size_t)env * PLEN_OBS;
+        io.nkey = obs_noise_base(seed, gid0 + env);
+    }
+    env_post<NOISE>(dc, sm.tab, ws, L, lane, io);
     store_record(state + (size_t)env * PLEN_STATE_WORDS, ws, L, lane);
 }
 
@@ -399,10 +445,12 @@ k_observe(const float *__restrict__ state, int n, float *__restrict__ obs) {
 }
 
 // PlenWalkEnv.reset (plen_env.py:558-614): copy the post-reset snapshot (or the robot's own row, rows != NULL) into the
-// selected envs
+// selected envs.  noise != NULL (plen_set_env_obs_noise): each reset robot draws its new episode's bias, obs receives the noisy
+// reset observation, clean_obs the clean one, and the robot's draw counter advances by one.
 __global__ void k_reset(float *__restrict__ state, int n, const uint8_t *__restrict__ mask,
                         const float *__restrict__ snap, float *__restrict__ obs, float *__restrict__ man,
-                        const float *__restrict__ rows) {
+                        const float *__restrict__ rows, float *__restrict__ noise, float *__restrict__ clean_obs,
+                        unsigned long long seed, long long gid0) {
     const int env = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (env >= n) return;
     if (mask && !mask[env]) return;
@@ -411,7 +459,24 @@ __global__ void k_reset(float *__restrict__ state, int n, const uint8_t *__restr
     rec[lane] = snapshot[lane];
     rec[32 + lane] = snapshot[32 + lane];
     rec[64 + lane] = snapshot[64 + lane];
-    if (obs && lane < PLEN_OBS) obs[(size_t)env * PLEN_OBS + lane] = snapshot[PLEN_STATE_WORDS + lane];
+    if (noise) {
+        float *nr = noise + (size_t)env * ON_WORDS;
+        const unsigned ctr = f_bits(nr[ON_CTR]);
+        const uint64_t key = obs_noise_base(seed, gid0 + env);
+        const float b = lane < 24 ? nr[ON_BETA + lane] * noise_normal(obs_noise_key(key, ctr, NS_BIAS, lane)) : 0.0f;
+        if (lane < PLEN_OBS) {
+            const float x = snapshot[PLEN_STATE_WORDS + lane];
+            clean_obs[(size_t)env * PLEN_OBS + lane] = x;
+            if (obs)
+                obs[(size_t)env * PLEN_OBS + lane] = obs_noise_word(x, lane, lane < 24 ? nr[ON_SIGMA + lane] : 0.0f, b, nr[ON_FLIP],
+                                                                    key, ctr, NS_ROBS);
+        }
+        __syncwarp();     // every lane has read the counter and its bias word
+        if (lane < 24) nr[ON_BIAS + lane] = b;
+        if (lane == 0) nr[ON_CTR] = bits_f(ctr + 1u);
+    } else if (obs && lane < PLEN_OBS) {
+        obs[(size_t)env * PLEN_OBS + lane] = snapshot[PLEN_STATE_WORDS + lane];
+    }
     if (man) {
         for (int w = lane; w < PLEN_MAN_WORDS; w += 32) man[(size_t)env * PLEN_MAN_WORDS + w] = snapshot[PLEN_SNAP_MAN + w];
     }
@@ -725,11 +790,20 @@ static void launch_step_range(plen_ctx *ctx, size_t off, int cnt, const float *a
     launch_ticks(ctx, state, cnt, actions_dev + off * PLEN_NJ, ctx->d_tgt + off * PLEN_NJ, ctx->cfg.substeps, st,
                  ctx->d_man ? ctx->d_man + off * PLEN_MAN_WORDS : nullptr, ev, off);
     if (ev) cudaEventRecord(ev[nev - 2], st);
-    k_post<<<dyn_grid(cnt), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->dc, ctx->d_tab, state, cnt, obs_dev + off * PLEN_OBS, reward_dev + off,
-                                                         done_dev + off, timeout_dev ? timeout_dev + off : nullptr,
-                                                         terminal_obs_dev ? terminal_obs_dev + off * PLEN_OBS : nullptr, ctx->d_snapshot,
-                                                         ctx->d_faults, ctx->d_man ? ctx->d_man + off * PLEN_MAN_WORDS : nullptr,
-                                                         ctx->d_rows ? ctx->d_rows + off * PLEN_SNAP_WORDS : nullptr);
+    float *man = ctx->d_man ? ctx->d_man + off * PLEN_MAN_WORDS : nullptr;
+    const float *rows = ctx->d_rows ? ctx->d_rows + off * PLEN_SNAP_WORDS : nullptr;
+    if (ctx->d_noise)
+        k_post<true><<<dyn_grid(cnt), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->dc, ctx->d_tab, state, cnt, obs_dev + off * PLEN_OBS, reward_dev + off,
+                                                                   done_dev + off, timeout_dev ? timeout_dev + off : nullptr,
+                                                                   terminal_obs_dev ? terminal_obs_dev + off * PLEN_OBS : nullptr,
+                                                                   ctx->d_snapshot, ctx->d_faults, man, rows, ctx->d_noise + off * ON_WORDS,
+                                                                   ctx->d_cobs + off * PLEN_OBS, ctx->d_ctobs + off * PLEN_OBS,
+                                                                   ctx->noise_seed, ctx->noise_first + (long long)off);
+    else
+        k_post<false><<<dyn_grid(cnt), DYN_WPC * 32, DYN_SMEM, st>>>(ctx->dc, ctx->d_tab, state, cnt, obs_dev + off * PLEN_OBS, reward_dev + off,
+                                                                    done_dev + off, timeout_dev ? timeout_dev + off : nullptr,
+                                                                    terminal_obs_dev ? terminal_obs_dev + off * PLEN_OBS : nullptr,
+                                                                    ctx->d_snapshot, ctx->d_faults, man, rows, nullptr, nullptr, nullptr, 0, 0);
     ctx->launches += 1;
     if (ev) cudaEventRecord(ev[nev - 1], st);
 }
@@ -760,7 +834,7 @@ unsigned long long plen_kernel_launches(const plen_ctx *ctx) { return ctx ? ctx-
 void plen_destroy(plen_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    cudaFree(ctx->d_tab); cudaFree(ctx->d_state); cudaFree(ctx->d_snapshot); cudaFree(ctx->d_srec); cudaFree(ctx->d_srx); cudaFree(ctx->d_xgroups); cudaFree(ctx->d_tgt); cudaFree(ctx->d_key); cudaFree(ctx->d_perm); cudaFree(ctx->d_scale); cudaFree(ctx->d_mass); cudaFree(ctx->d_lat); cudaFree(ctx->d_rows); cudaFree(ctx->d_rscr); cudaFree(ctx->d_man); cudaFree(ctx->d_hull);
+    cudaFree(ctx->d_tab); cudaFree(ctx->d_state); cudaFree(ctx->d_snapshot); cudaFree(ctx->d_srec); cudaFree(ctx->d_srx); cudaFree(ctx->d_xgroups); cudaFree(ctx->d_tgt); cudaFree(ctx->d_key); cudaFree(ctx->d_perm); cudaFree(ctx->d_scale); cudaFree(ctx->d_mass); cudaFree(ctx->d_lat); cudaFree(ctx->d_rows); cudaFree(ctx->d_rscr); cudaFree(ctx->d_noise); cudaFree(ctx->d_cobs); cudaFree(ctx->d_ctobs); cudaFree(ctx->d_man); cudaFree(ctx->d_hull);
     cudaFree(ctx->d_act); cudaFree(ctx->d_obs); cudaFree(ctx->d_rew); cudaFree(ctx->d_done); cudaFree(ctx->d_tmo); cudaFree(ctx->d_faults);
     for (int k = 1; k < PLEN_HOST_PIPE; k++)
         if (ctx->pipe[k]) cudaStreamDestroy(ctx->pipe[k]);
@@ -792,7 +866,8 @@ static int create_impl(plen_ctx *ctx) {
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaFuncSetAttribute(k_dyn<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_dyn<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
-    CK(ctx, cudaFuncSetAttribute(k_post, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
+    CK(ctx, cudaFuncSetAttribute(k_post<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
+    CK(ctx, cudaFuncSetAttribute(k_post<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_observe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_pack_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DYN_SMEM));
     CK(ctx, cudaFuncSetAttribute(k_solve<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SOLVE_SMEM));
@@ -850,7 +925,8 @@ static int create_impl(plen_ctx *ctx) {
     launch_ticks(ctx, ctx->d_snapshot, 1, nullptr, nullptr, ctx->cfg.reset_ticks, ctx->stream,
                  ctx->d_man ? ctx->d_snapshot + PLEN_SNAP_MAN : nullptr);
     k_observe<<<1, 32, DYN_SMEM, ctx->stream>>>(ctx->d_snapshot, 1, ctx->d_snapshot + PLEN_STATE_WORDS);
-    k_reset<<<(n * 32 + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_state, n, nullptr, ctx->d_snapshot, nullptr, ctx->d_man, nullptr);
+    k_reset<<<(n * 32 + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_state, n, nullptr, ctx->d_snapshot, nullptr, ctx->d_man, nullptr,
+                                                          nullptr, nullptr, 0, 0);
     CK(ctx, cudaGetLastError());
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return PLEN_OK;
@@ -890,7 +966,8 @@ int plen_reset(plen_ctx *ctx, const uint8_t *mask_dev, float *obs_dev, void *str
     if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
     CK(ctx, cudaSetDevice(ctx->device));
     k_reset<<<(ctx->n * 32 + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ctx->d_state, ctx->n, mask_dev, ctx->d_snapshot, obs_dev, ctx->d_man,
-                                                                       ctx->d_rows);
+                                                                       ctx->d_rows, ctx->d_noise, ctx->d_cobs, ctx->noise_seed,
+                                                                       ctx->noise_first);
     ctx->launches += 1;
     CK(ctx, cudaGetLastError());
     CK(ctx, mark_work(ctx, (cudaStream_t)stream));
@@ -979,7 +1056,8 @@ int plen_step_host(plen_ctx *ctx, const float *actions_host, float *obs_host, fl
         cudaStream_t st = ctx->pipe[used % PLEN_HOST_PIPE];
         // ordering contract (plen_b200.h): this call runs on the context's private streams, so it first waits for whatever
         // the last stream-taking entry point (reset / step / set_state / set_env_scales / set_env_mass / set_env_latency /
-        // settle_env_resets / set_env_resets / clear_env_resets / tick) queued on the caller's stream
+        // settle_env_resets / set_env_resets / clear_env_resets / set_env_obs_noise / set_env_obs_noise_state /
+        // clear_env_obs_noise / tick) queued on the caller's stream
         CK(ctx, cudaStreamWaitEvent(st, ctx->last_work, 0));
         CK(ctx, cudaMemcpyAsync(ctx->d_act + off * PLEN_NJ, actions_host + off * PLEN_NJ, sizeof(float) * PLEN_NJ * cnt,
                                 cudaMemcpyHostToDevice, st));
@@ -1164,6 +1242,92 @@ int plen_clear_env_resets(plen_ctx *ctx, void *stream) {
     ctx->d_rows = ctx->d_rscr = nullptr;
     CK(ctx, e0 != cudaSuccess ? e0 : e1);
     CK(ctx, mark_work(ctx, (cudaStream_t)stream));
+    return PLEN_OK;
+}
+
+int plen_set_env_obs_noise(plen_ctx *ctx, const float *sigma_dev, const float *bias_std_dev, const float *flip_dev,
+                           unsigned long long seed, long long first_env_id, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    if (first_env_id < 0) return fail(ctx, PLEN_E_ARG, "plen_set_env_obs_noise: first_env_id %lld < 0", first_env_id);
+    CK(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t n = ctx->n, words = (size_t)ON_WORDS * n;
+    const int init = !ctx->d_noise;         // the rows are allocated at the first call: a context that never sets them has none
+    if (init) {
+        cudaError_t e = cudaMalloc(&ctx->d_noise, sizeof(float) * words);
+        if (e == cudaSuccess) e = cudaMalloc(&ctx->d_cobs, sizeof(float) * PLEN_OBS * n);
+        if (e == cudaSuccess) e = cudaMalloc(&ctx->d_ctobs, sizeof(float) * PLEN_OBS * n);
+        if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_cobs, 0, sizeof(float) * PLEN_OBS * n, st);
+        if (e == cudaSuccess) e = cudaMemsetAsync(ctx->d_ctobs, 0, sizeof(float) * PLEN_OBS * n, st);
+        if (e != cudaSuccess) {
+            cudaFree(ctx->d_noise); cudaFree(ctx->d_cobs); cudaFree(ctx->d_ctobs);
+            ctx->d_noise = ctx->d_cobs = ctx->d_ctobs = nullptr;
+            return fail(ctx, PLEN_E_CUDA, "plen_set_env_obs_noise: %s", cudaGetErrorString(e));
+        }
+    }
+    k_set_obs_noise<<<(unsigned)((words + 255) / 256), 256, 0, st>>>(ctx->d_noise, ctx->n, sigma_dev, bias_std_dev, flip_dev, nullptr,
+                                                                     nullptr, init);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        if (init) {     // rows that were never zeroed must never be stepped with
+            cudaFree(ctx->d_noise); cudaFree(ctx->d_cobs); cudaFree(ctx->d_ctobs);
+            ctx->d_noise = ctx->d_cobs = ctx->d_ctobs = nullptr;
+        }
+        return fail(ctx, PLEN_E_CUDA, "plen_set_env_obs_noise: k_set_obs_noise: %s", cudaGetErrorString(e));
+    }
+    ctx->noise_seed = seed;
+    ctx->noise_first = first_env_id;
+    CK(ctx, mark_work(ctx, st));
+    return PLEN_OK;
+}
+
+int plen_set_env_obs_noise_state(plen_ctx *ctx, const float *bias_dev, const uint32_t *counter_dev, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    if (!ctx->d_noise) return fail(ctx, PLEN_E_STATE, "plen_set_env_obs_noise_state: no noise table (call plen_set_env_obs_noise first)");
+    CK(ctx, cudaSetDevice(ctx->device));
+    const size_t words = (size_t)ON_WORDS * ctx->n;
+    k_set_obs_noise<<<(unsigned)((words + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ctx->d_noise, ctx->n, nullptr, nullptr, nullptr,
+                                                                                      bias_dev, counter_dev, 0);
+    CK(ctx, cudaGetLastError());
+    CK(ctx, mark_work(ctx, (cudaStream_t)stream));
+    return PLEN_OK;
+}
+
+int plen_get_env_obs_noise(plen_ctx *ctx, float *sigma_dev, float *bias_std_dev, float *flip_dev, float *bias_dev,
+                           uint32_t *counter_dev, unsigned long long *seed, long long *first_env_id, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    CK(ctx, cudaSetDevice(ctx->device));
+    const size_t words = (size_t)ON_WORDS * ctx->n;
+    if (sigma_dev || bias_std_dev || flip_dev || bias_dev || counter_dev)
+        k_get_obs_noise<<<(unsigned)((words + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ctx->d_noise, ctx->n, sigma_dev, bias_std_dev,
+                                                                                          flip_dev, bias_dev, counter_dev);
+    CK(ctx, cudaGetLastError());
+    if (seed) *seed = ctx->d_noise ? ctx->noise_seed : 0;
+    if (first_env_id) *first_env_id = ctx->d_noise ? ctx->noise_first : 0;
+    return ctx->d_noise ? 1 : 0;
+}
+
+int plen_clear_env_obs_noise(plen_ctx *ctx, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    if (!ctx->d_noise) return PLEN_OK;
+    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, cudaStreamSynchronize((cudaStream_t)stream));     // steps queued before this call still use the rows
+    const cudaError_t e0 = cudaFree(ctx->d_noise), e1 = cudaFree(ctx->d_cobs), e2 = cudaFree(ctx->d_ctobs);
+    ctx->d_noise = ctx->d_cobs = ctx->d_ctobs = nullptr;
+    ctx->noise_seed = 0;
+    ctx->noise_first = 0;
+    CK(ctx, e0 != cudaSuccess ? e0 : e1 != cudaSuccess ? e1 : e2);
+    CK(ctx, mark_work(ctx, (cudaStream_t)stream));
+    return PLEN_OK;
+}
+
+int plen_get_clean_obs(plen_ctx *ctx, float *obs_dev, float *terminal_obs_dev, void *stream) {
+    if (!ctx) return fail(nullptr, PLEN_E_ARG, "ctx is NULL");
+    if (!ctx->d_noise) return fail(ctx, PLEN_E_STATE, "plen_get_clean_obs: no noise table (the observations are the clean ones)");
+    CK(ctx, cudaSetDevice(ctx->device));
+    const size_t bytes = sizeof(float) * PLEN_OBS * (size_t)ctx->n;
+    if (obs_dev) CK(ctx, cudaMemcpyAsync(obs_dev, ctx->d_cobs, bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    if (terminal_obs_dev) CK(ctx, cudaMemcpyAsync(terminal_obs_dev, ctx->d_ctobs, bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return PLEN_OK;
 }
 

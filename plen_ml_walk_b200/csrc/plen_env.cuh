@@ -103,7 +103,65 @@ struct StepIO {
     const float *snapshot;    // [96 + 26] post-reset record and its observation: the shared snapshot or the robot's own reset row
     unsigned long long *faults;   // device counter of numeric faults (nullable)
     float *man;               // this robot's persistent sole manifold (sole_manifold = 1), nullable: reset with the record
+    // observation noise (plen_set_env_obs_noise; read by env_post<true> only)
+    float *noise;             // [ON_WORDS] this robot's noise row
+    float *clean_obs;         // [26] the noise-free obs
+    float *clean_tobs;        // [26] the noise-free terminal obs, written where done
+    unsigned long long nkey;  // obs_noise_base(seed, first_env_id + robot)
 };
+
+// ---- observation noise (plen_set_env_obs_noise) ------------------------------------------------------------------
+// Noise row of a robot, ON_WORDS floats: sigma [24] | bias std beta [24] | bias b of the running episode [24] | flip p | draw
+// counter (uint32 bits) | padding.  Continuous words w = 0..23 of an observation the agent receives become
+//   clean_w + fmaf(sigma_w, n, b_w)   (passed through bit for bit where sigma_w == 0 and b_w == 0),
+// contact flags w = 24, 25 become 1 - clean_w with probability p.  No clipping, no angle wrapping.  b_w = beta_w * n' is drawn
+// at every reset of the robot and kept for its episode.  Draws are counter-based:
+//   key(w, s) = mix64(seed ^ mix64(gid)) + (counter << 8) + (s << 5) + w       (uint64 arithmetic, gid = first_env_id + robot)
+//   hash32(k) = mix64(k) >> 32,  mix64 = the splitmix64 finaliser (x += 0x9E3779B97F4A7C15, then the two xor-shift-multiplies
+//               and the final x ^ (x >> 31))
+//   n = sqrtf(-2 logf(u1)) * cospif(2 u2),  u1 = ((float)hash32(k) + 1) * 2.3283064e-10f,
+//       u2 = (float)hash32(k ^ 0xA5A5A5A5DEADBEEF) * 2.3283064e-10f                  (the generator of plen_actor_forward)
+//   flip where (uint64)hash32(k) < (uint64)((double)p * 2^32)                       (p = 0 never flips, p = 1 always)
+// Streams s: the step's obs noise, its flips, the new episode's bias, the reset obs noise, its flips.  k_post draws with the
+// counter and then increments it once; k_reset does the same once per robot it resets.
+enum { ON_SIGMA = 0, ON_BETA = 24, ON_BIAS = 48, ON_FLIP = 72, ON_CTR = 73, ON_WORDS = 96 };
+enum { NS_OBS = 0, NS_FLIP = 1, NS_BIAS = 2, NS_ROBS = 3, NS_RFLIP = 4 };
+
+PLEN_DEV uint64_t mix64(uint64_t x) {
+    x += 0x9E3779B97F4A7C15ull;
+    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
+    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
+    return x ^ (x >> 31);
+}
+PLEN_DEV uint32_t noise_hash32(uint64_t k) { return (uint32_t)(mix64(k) >> 32); }
+PLEN_DEV uint64_t obs_noise_base(unsigned long long seed, long long gid) { return mix64(seed ^ mix64((uint64_t)gid)); }
+PLEN_DEV uint64_t obs_noise_key(uint64_t base, unsigned ctr, int stream, int word) {
+    return base + ((uint64_t)ctr << 8) + ((uint64_t)stream << 5) + (uint64_t)word;
+}
+// float with the given bit pattern (the inverse of f_bits): the draw counter travels in a float word of the noise row
+#ifndef PLEN_HOST_EMU
+PLEN_DEV float bits_f(unsigned u) { return __uint_as_float(u); }
+#else
+PLEN_DEV float bits_f(unsigned u) { float32_t_ f; std::memcpy(&f, &u, 4); return (float)f; }
+#endif
+PLEN_DEV float noise_u1(uint64_t k) { return ((float)noise_hash32(k) + 1.0f) * 2.3283064e-10f; }
+PLEN_DEV float noise_u2(uint64_t k) { return (float)noise_hash32(k ^ 0xA5A5A5A5DEADBEEFull) * 2.3283064e-10f; }
+PLEN_DEV float noise_normal(uint64_t k) {
+    const float u1 = noise_u1(k), u2 = noise_u2(k);
+#ifndef PLEN_HOST_EMU
+    return sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);
+#else   // the host has no cospif: libm in double, rounded to the build's precision
+    return (float)(std::sqrt(-2.0 * std::log((double)u1)) * std::cos(3.14159265358979323846 * (double)(2.0f * u2)));
+#endif
+}
+PLEN_DEV bool noise_flip(uint64_t k, float p) { return (uint64_t)noise_hash32(k) < (uint64_t)((double)p * 4294967296.0); }
+
+// one observation word through the noise of its lane: a continuous word (lane < 24) with sigma, b and the Gaussian of stream
+// s, a contact flag (lanes 24, 25) with flip probability p and stream s + 1
+PLEN_DEV float obs_noise_word(float x, int lane, float sigma, float b, float p, uint64_t base, unsigned ctr, int s) {
+    if (lane < 24) return (sigma == 0.0f && b == 0.0f) ? x : x + fmaf(sigma, noise_normal(obs_noise_key(base, ctr, s, lane)), b);
+    return noise_flip(obs_noise_key(base, ctr, s + 1, lane), p) ? 1.0f - x : x;
+}
 
 // env_ranges of plen_env.py:148-167 are kept in double so that the a = +-1 inset branch (plen_env.py:707-711) takes
 // the same side as the reference's float64 arithmetic.
@@ -133,6 +191,9 @@ PLEN_DEV int latency_source(int d, int k, int S, int ep_t) {
 PLEN_DEV int latency_slot(int ep_t, int s) { return (ep_t + LAT_SLOTS - s) % LAT_SLOTS; }
 
 // Everything of PlenWalkEnv.step after the 4 physics ticks (:671-678) + TimeLimit + optional auto-reset (k_post).
+// NOISE: observation noise at the obs / terminal_obs stores (io.noise), the clean words into io.clean_obs / io.clean_tobs;
+// everything else -- reward, done, counters, the record -- is the stock computation on the true state.
+template <bool NOISE = false>
 PLEN_DEV void env_post(const DevConfig &cfg, const float *tab, WarpScratch &ws, LaneState &L, int lane,
                        const StepIO &io) {
     // ---- compute_observation (:768-871)
@@ -237,7 +298,42 @@ PLEN_DEV void env_post(const DevConfig &cfg, const float *tab, WarpScratch &ws, 
         ws.st[W_SUMS + (lane - 6)] = v;
     }
     warp_sync();
-    if ((done && cfg.auto_reset) || fault) {
+    if constexpr (NOISE) {
+        // this lane's noise parameters: sigma, b of the running episode and beta for words 0..23, p for the flags
+        const float *nr = io.noise;
+        const unsigned ctr = f_bits(nr[ON_CTR]);
+        const float sigma = lane < 24 ? nr[ON_SIGMA + lane] : 0.0f, b = lane < 24 ? nr[ON_BIAS + lane] : 0.0f;
+        const float beta = lane < 24 ? nr[ON_BETA + lane] : 0.0f, p = nr[ON_FLIP];
+        const float x = lane < 26 ? ws.obs[lane] : 0.0f;
+        if ((done && cfg.auto_reset) || fault) {
+            const float tx = (lane < 26 && fault) ? io.snapshot[96 + lane] : x;
+            if (lane < 26) {      // the finished episode's terminal observation carries its own bias
+                io.clean_tobs[lane] = tx;
+                if (io.terminal_obs) io.terminal_obs[lane] = obs_noise_word(tx, lane, sigma, b, p, io.nkey, ctr, NS_OBS);
+            }
+            load_record(io.snapshot, ws, L, lane);
+            const float nb = lane < 24 ? beta * noise_normal(obs_noise_key(io.nkey, ctr, NS_BIAS, lane)) : 0.0f;
+            if (lane < 26) {
+                const float rx = io.snapshot[96 + lane];
+                io.clean_obs[lane] = rx;
+                io.obs[lane] = obs_noise_word(rx, lane, sigma, nb, p, io.nkey, ctr, NS_ROBS);
+            }
+            if (lane < 24) io.noise[ON_BIAS + lane] = nb;
+            if (io.man) {
+                for (int w = lane; w < PLEN_MAN_WORDS; w += 32) io.man[w] = io.snapshot[PLEN_SNAP_MAN + w];
+            }
+        } else if (lane < 26) {
+            const float y = obs_noise_word(x, lane, sigma, b, p, io.nkey, ctr, NS_OBS);
+            io.clean_obs[lane] = x;
+            io.obs[lane] = y;
+            if (done) {
+                io.clean_tobs[lane] = x;
+                if (io.terminal_obs) io.terminal_obs[lane] = y;
+            }
+        }
+        warp_sync();      // every lane has read the counter
+        if (lane == 0) io.noise[ON_CTR] = bits_f(ctr + 1u);
+    } else if ((done && cfg.auto_reset) || fault) {
         // the reference caller resets after a terminal step (plen_td3.py:122-129); the reset is deterministic
         // (fixed pose + 8 ticks, plen_env.py:561-570) so the post-reset record is precomputed: the shared snapshot, or the
         // robot's own row settled under its parameters (plen_settle_env_resets)

@@ -25,6 +25,9 @@ from . import _abi
 from .urdf_loader import PlenModel, packaged_model
 
 OBS_DIM, ACT_DIM = 26, 18
+# the observation words (plen_env.py:816-822); set_obs_noise's std / bias_std cover the first 24, contact_flip the last two
+OBS_NAMES = ["q%d" % (j + 1) for j in range(18)] + ["z", "vx", "roll", "pitch", "yaw", "y", "right_contact", "left_contact"]
+NOISE_WORDS = 24
 
 # plen_env.py:148-167 (env_ranges) and :170-189 (real_ranges)
 ENV_RANGES = [[-1.57, 1.57], [-0.15, 1.5], [-0.95, 0.75], [-0.9, 0.3], [-0.95, 1.2], [-0.8, 0.4],
@@ -96,6 +99,8 @@ class PlenVecEnv:
         self._done = torch.empty(n, dtype=torch.uint8, device=dev)
         self._timeout = torch.empty(n, dtype=torch.uint8, device=dev)
         self._scales = {}                                                  # per-env scales set so far (set_env_scales)
+        self._noise_on = False                                             # set_obs_noise called (and not cleared)
+        self._clean_obs = self._clean_terminal_obs = None
 
     # ---- plumbing
     def _check(self, rc):
@@ -143,6 +148,8 @@ class PlenVecEnv:
                                            self._p(self._done), self._p(self._timeout), self._p(self._terminal_obs),
                                            self._stream()))
         info = {"terminal_obs": self._terminal_obs, "timeout": self._timeout.bool()}
+        if self._noise_on:
+            info["clean_obs"], info["clean_terminal_obs"] = self.clean_obs()
         return self._obs, self._reward, self._done.bool(), info
 
     def step_host(self, actions_host, obs_host, reward_host, done_host, timeout_host=None):
@@ -389,19 +396,135 @@ class PlenVecEnv:
         with torch.cuda.device(self.device):
             self._check(self.lib.plen_clear_env_resets(self._ctx, self._stream()))
 
+    def _noise_param(self, x, name):
+        """float, [24], [N] or [N,24] (a 1-D [24] is per word, also when N == 24) -> [N,24] float32 on the device"""
+        n = self.num_envs
+        t = torch.as_tensor(x, dtype=torch.float32, device=self.device)
+        if t.dim() == 0:
+            t = t.expand(n, NOISE_WORDS)
+        elif tuple(t.shape) == (NOISE_WORDS,):
+            t = t[None, :].expand(n, NOISE_WORDS)
+        elif tuple(t.shape) == (n,):
+            t = t[:, None].expand(n, NOISE_WORDS)
+        if tuple(t.shape) != (n, NOISE_WORDS):
+            raise ValueError("%s: expected a float, (%d,), (%d,) or (%d, %d), got %s" % (name, NOISE_WORDS, n, n, NOISE_WORDS,
+                                                                                       tuple(t.shape)))
+        if not bool(torch.isfinite(t).all()) or not bool((t >= 0).all()):
+            raise ValueError("%s must be finite and >= 0" % name)
+        return t.contiguous()
+
+    def set_obs_noise(self, std=None, bias_std=None, contact_flip=None, seed=None, first_env_id=None):
+        """Per-env observation noise (SURVEY.md 8f-3, sensing side): what step() / step_host() / reset() return as obs and
+        info["terminal_obs"] carries sensor noise; reward, done, the gait counters and the physics keep the true state.
+
+        std:          white noise sigma of the 24 continuous words (OBS_NAMES[:24]: q1..q18 rad, z m, vx m/s, roll / pitch /
+                      yaw rad, y m): a float, [24] (per word), [N] (per robot) or [N,24].  Fresh N(0, sigma^2) every observation.
+        bias_std:     the same shapes: std of a per-episode bias b = bias_std * N(0,1), drawn at every reset of the robot and
+                      constant over its episode (IMU offset, servo zero error).  Episodes running at the first call keep b = 0.
+        contact_flip: a float or [N]: probability that each contact flag (OBS_NAMES[24:]) reads 1 - flag.
+        seed:         of the counter-based draws (default: the current one, 0 at the first call).
+        first_env_id: global id of robot 0 (default: the current one, 0): a shard of a larger population passes its first
+                      robot's id and draws the noise that robot would get in one big env.
+        None leaves a part unchanged (zero at the first call).  Words with std = bias = 0 are passed through bit for bit.  No
+        clipping or angle wrapping is applied.  Raises ValueError on a wrong shape, a non-finite or negative std, a
+        contact_flip outside [0, 1], or a negative first_env_id.  While noise is on, step() adds info["clean_obs"] and
+        info["clean_terminal_obs"] (clean_obs()).  The draws advance with a counter on the device, so a captured CUDA graph
+        of step() draws new noise on every replay."""
+        n = self.num_envs
+        s = None if std is None else self._noise_param(std, "std")
+        b = None if bias_std is None else self._noise_param(bias_std, "bias_std")
+        f = None
+        if contact_flip is not None:
+            f = torch.as_tensor(contact_flip, dtype=torch.float32, device=self.device)
+            if f.dim() == 0:
+                f = f.expand(n)
+            f = self._dev_f32(f, (n,))
+            if not bool(torch.isfinite(f).all()) or not bool(((f >= 0) & (f <= 1)).all()):
+                raise ValueError("contact_flip must lie in [0, 1]")
+        _, cur_seed, cur_first = self._get_obs_noise_params()
+        seed = cur_seed if seed is None else int(seed)
+        first = cur_first if first_env_id is None else int(first_env_id)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("seed must lie in 0 .. 2^64 - 1")
+        if first < 0:
+            raise ValueError("first_env_id must be >= 0")
+        with torch.cuda.device(self.device):
+            self._check(self.lib.plen_set_env_obs_noise(self._ctx, self._p(s), self._p(b), self._p(f), C.c_ulonglong(seed),
+                                                        C.c_longlong(first), self._stream()))
+        self._noise_on = True
+        if self._clean_obs is None:     # allocated here, not inside a step that may be under CUDA graph capture
+            self._clean_obs = torch.zeros((n, OBS_DIM), dtype=torch.float32, device=self.device)
+            self._clean_terminal_obs = torch.zeros((n, OBS_DIM), dtype=torch.float32, device=self.device)
+
+    def _get_obs_noise_params(self):
+        seed, first = C.c_ulonglong(), C.c_longlong()
+        rc = self.lib.plen_get_env_obs_noise(self._ctx, None, None, None, None, None, C.byref(seed), C.byref(first), self._stream())
+        if rc < 0:
+            self._check(rc)
+        return rc == 1, int(seed.value), int(first.value)
+
+    def get_obs_noise(self):
+        """-> dict(std [N,24], bias_std [N,24], contact_flip [N], bias [N,24] of the running episodes, counter [N] int32
+        (the draw counters' uint32 bits), seed, first_env_id, active); zeros where set_obs_noise was never called."""
+        n, dev = self.num_envs, self.device
+        s, b, bias = (torch.empty((n, NOISE_WORDS), dtype=torch.float32, device=dev) for _ in range(3))
+        f = torch.empty(n, dtype=torch.float32, device=dev)
+        c = torch.empty(n, dtype=torch.int32, device=dev)
+        seed, first = C.c_ulonglong(), C.c_longlong()
+        with torch.cuda.device(self.device):
+            rc = self.lib.plen_get_env_obs_noise(self._ctx, self._p(s), self._p(b), self._p(f), self._p(bias), self._p(c),
+                                                 C.byref(seed), C.byref(first), self._stream())
+        if rc < 0:
+            self._check(rc)
+        return {"std": s, "bias_std": b, "contact_flip": f, "bias": bias, "counter": c, "seed": int(seed.value),
+                "first_env_id": int(first.value), "active": rc == 1}
+
+    def set_obs_noise_state(self, bias=None, counter=None):
+        """The running per-episode biases [N,24] and draw counters [N] (uint32 bits, as get_obs_noise returns them); for
+        snapshots that continue a noisy run bit for bit.  Needs set_obs_noise first."""
+        n = self.num_envs
+        b = None if bias is None else self._dev_f32(bias, (n, NOISE_WORDS))
+        c = None
+        if counter is not None:
+            c = torch.as_tensor(counter, device=self.device)
+            if tuple(c.shape) != (n,):
+                raise ValueError("counter: expected shape (%d,), got %s" % (n, tuple(c.shape)))
+            c = c.to(torch.int32).contiguous() if c.dtype != torch.int64 else \
+                torch.where(c >= 2 ** 31, c - 2 ** 32, c).to(torch.int32).contiguous()
+        with torch.cuda.device(self.device):
+            self._check(self.lib.plen_set_env_obs_noise_state(self._ctx, self._p(b), self._p(c), self._stream()))
+
+    def clear_obs_noise(self):
+        """Switch the observation noise off: the env is exactly the stock path again."""
+        with torch.cuda.device(self.device):
+            self._check(self.lib.plen_clear_env_obs_noise(self._ctx, self._stream()))
+        self._noise_on = False
+
+    def clean_obs(self):
+        """-> (obs [N,26], terminal_obs [N,26]): the noise-free observations of the last step or reset, and the noise-free
+        terminal observations (written where a step reported done).  Reused buffers.  Needs set_obs_noise."""
+        if self._clean_obs is None:
+            raise RuntimeError("clean_obs: observation noise is off (call set_obs_noise first); obs is the clean observation")
+        with torch.cuda.device(self.device):
+            self._check(self.lib.plen_get_clean_obs(self._ctx, self._p(self._clean_obs), self._p(self._clean_terminal_obs),
+                                                    self._stream()))
+        return self._clean_obs, self._clean_terminal_obs
+
     def save_state(self, path):
         """Snapshot of every env (pose, velocities, contact cache, env bookkeeping, per-env scales, masses, command delays,
-        command history and reset states) to one .pt file (SURVEY.md 8f-4)."""
+        command history, reset states and observation noise) to one .pt file (SURVEY.md 8f-4)."""
         qpos, qvel, aux = self.get_state()
         ms, mp, mass_set = self._get_env_mass()
         lt, lh, lat_set = self._get_env_latency()
         rows, rows_set = self._get_env_resets()
+        nz = self.get_obs_noise()
         torch.save({"num_envs": self.num_envs, "joint_act": self.joint_act, "qpos": qpos.cpu(), "qvel": qvel.cpu(), "aux": aux.cpu(),
                     "scales": {k: v.cpu() for k, v in self._scales.items()},
                     "mass": {"scale": ms.cpu(), "payload": mp.cpu()} if mass_set else None,
                     "latency": {"ticks": lt.cpu(), "history": lh.cpu()} if lat_set else None,
                     "resets": dict(zip(("qpos", "qvel", "aux", "man"), (None if t is None else t.cpu() for t in rows[:3] + rows[4:])))
                     if rows_set else None,
+                    "obs_noise": {k: (v.cpu() if isinstance(v, torch.Tensor) else v) for k, v in nz.items()} if nz["active"] else None,
                     "manifold": self.get_manifold().cpu() if int(self.cfg.sole_manifold) else None}, path)
 
     def load_state(self, path):
@@ -431,6 +554,12 @@ class PlenVecEnv:
             self.set_env_resets(rows["qpos"], rows["qvel"], rows["aux"], rows["man"])
         else:
             self.clear_env_resets()
+        nz = d.get("obs_noise")
+        if nz is not None:          # parameters, running biases and draw counters: the noisy run continues bit for bit
+            self.set_obs_noise(nz["std"], nz["bias_std"], nz["contact_flip"], seed=nz["seed"], first_env_id=nz["first_env_id"])
+            self.set_obs_noise_state(nz["bias"], nz["counter"])
+        else:
+            self.clear_obs_noise()
 
     def tick(self, targets, n_ticks=1):
         """Raw physics: n_ticks of 1/240 s with joint targets in radians, no env logic (move_joints + stepSimulation)."""

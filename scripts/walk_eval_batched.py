@@ -11,6 +11,8 @@ noise to give a distribution.  Reports episode length / return of the first epis
     python scripts/walk_eval_batched.py [--envs 4096] [--sigma 0.05] [--precision fp32|fp16]
                                         [--mass-scale S] [--payload KG [--payload-offset X Y Z]] [--latency-ticks D | LO:HI]
                                         [--settle-resets] [--start-pose X Y Z YAW]
+                                        [--obs-noise-joints RAD] [--obs-noise-imu RAD] [--obs-noise-vx MPS] [--obs-noise-base M]
+                                        [--obs-bias-joints RAD] [--obs-bias-imu RAD] [--contact-flip P]
 
 --mass-scale / --payload sweep the policy's robustness to the robot's mass (PlenVecEnv.set_env_mass): every body x S, and a
 point mass of KG kg on the torso, by default at the torso body's centre of mass.  --latency-ticks sweeps its robustness to servo
@@ -22,6 +24,12 @@ latency setters, before reset()); without it a robot starts from the one snapsho
 --start-pose settles every robot from base position (X, Y, Z) with heading YAW about world z instead of the reference's start
 (implies --settle-resets).  The distance walked is reported as the distance of the base from its settled start position in the
 ground plane, alongside the final x.
+
+--obs-noise-* / --obs-bias-* / --contact-flip sweep the policy's robustness to sensor noise (PlenVecEnv.set_obs_noise): white
+noise of that std on the joint angles, on roll / pitch / yaw (the IMU), on vx, on z and y (the base position); a per-episode
+bias of that std on the joint angles or the IMU; each contact flag read wrong with probability P.  The policy acts on the noisy
+observations; reward, termination and the distances are the true ones.  Env 0 keeps a zero noise row: it stays the
+noise-free deterministic rollout.
 """
 import argparse
 import json
@@ -58,6 +66,9 @@ def main():
                     help="settle each robot's reset state under its own masses and scales before the rollouts")
     ap.add_argument("--start-pose", type=float, nargs=4, default=None, metavar=("X", "Y", "Z", "YAW"),
                     help="start every robot from this base position (m) and heading (rad); implies --settle-resets")
+    for flag, what in (("--obs-noise-joints", "RAD"), ("--obs-noise-imu", "RAD"), ("--obs-noise-vx", "MPS"), ("--obs-noise-base", "M"),
+                       ("--obs-bias-joints", "RAD"), ("--obs-bias-imu", "RAD"), ("--contact-flip", "P")):
+        ap.add_argument(flag, type=float, default=0.0, metavar=what, help="observation noise (see the module docstring)")
     a = ap.parse_args()
     dev = torch.device("cuda:0")
     g = np.load(GOLD)
@@ -82,6 +93,20 @@ def main():
         gen = torch.Generator(device=dev); gen.manual_seed(0)
         env.set_env_latency(torch.randint(lo, hi + 1, (n,), device=dev, generator=gen))
         latency = {"ticks_lo": lo, "ticks_hi": hi, "ms_per_tick": 1000.0 * float(env.cfg.dt)}
+    obs_noise = None
+    groups = {"joints": range(0, 18), "imu": range(20, 23), "vx": [19], "base": [18, 23]}
+    if any(getattr(a, k) for k in ("obs_noise_joints", "obs_noise_imu", "obs_noise_vx", "obs_noise_base", "obs_bias_joints",
+                                   "obs_bias_imu", "contact_flip")):
+        std, bias = torch.zeros(n, 24), torch.zeros(n, 24)
+        for gname, words in groups.items():
+            std[1:, list(words)] = getattr(a, "obs_noise_" + gname)
+            if gname in ("joints", "imu"):
+                bias[1:, list(words)] = getattr(a, "obs_bias_" + gname)
+        flip = torch.full((n,), a.contact_flip)
+        flip[0] = 0.0                                                        # env 0: the noise-free deterministic rollout
+        env.set_obs_noise(std, bias, flip, seed=0)
+        obs_noise = {k: getattr(a, k) for k in ("obs_noise_joints", "obs_noise_imu", "obs_noise_vx", "obs_noise_base",
+                                                "obs_bias_joints", "obs_bias_imu", "contact_flip")}
     settle = a.settle_resets or a.start_pose is not None
     if settle:
         env.settle_resets(start_pose=a.start_pose)
@@ -106,6 +131,7 @@ def main():
     print(json.dumps({
         "policy": "plen_walk_gazebo_3229999 (reference checkpoint)", "envs": n, "steps": a.steps, "sigma": a.sigma,
         "precision": a.precision, "sole_manifold": a.sole_manifold, "config_overrides": ovr, "mass": mass, "latency": latency,
+        "obs_noise": obs_noise,
         "settled_resets": settle, "start_pose": a.start_pose,
         "deterministic": {"episode_length": float(L[0]), "return": float(R[0]), "x_final_m": float(X[0]),
                           "distance_from_start_m": float(D[0])},
